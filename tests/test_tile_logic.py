@@ -47,18 +47,23 @@ def packed_lut():
 LUT = packed_lut()
 
 
+OUT_DTYPES = {_capi.OUT_CAM_F32: np.float32, _capi.OUT_LIN_F32: np.float32, _capi.OUT_LIN_F16: np.float16,
+              _capi.OUT_SRGB_U8: np.uint8, _capi.OUT_SRGB_U16: np.uint16}
+
+
 def emu_develop(lib, src, stages, pattern="RGGB", tile=(16, 8), black=syn.BLACK, white=syn.WHITE,
-                out_kind=_capi.OUT_LIN_F32, band=None, hdr=False, held=None, quality=0):
+                out_kind=_capi.OUT_LIN_F32, band=None, hdr=False, held=None, quality=0, gamma=False):
     """src: uint16 counts or float32 sensor; `held` = (row0, rows) keeps only that slice of the frame."""
     H, W = src.shape
     rb, re = band or (0, H)
-    out = np.full((re - rb, W, 3), np.nan, dtype=np.float32)
+    dt = OUT_DTYPES[out_kind]
+    out = np.full((re - rb, W, 3), np.nan if dt == np.float32 else 0xA5, dtype=dt)
     nscr = (2 if stages >= 2 else 1) * ((re - rb) + 8 * max(stages, 0)) * W * 3
     scratch = np.full(max(nscr, 1), np.nan, dtype=np.float32)
     r0, nr = held or (0, H)
     part = np.ascontiguousarray(src[r0:r0 + nr])
     a = _capi.fill_develop_args(H, W, pattern, _capi.IN_U16 if src.dtype == np.uint16 else _capi.IN_F32,
-                                part.ctypes.data, part.strides[0], r0, nr, black, white, WB, M, stages, hdr, False,
+                                part.ctypes.data, part.strides[0], r0, nr, black, white, WB, M, stages, hdr, gamma,
                                 out_kind, out.ctypes.data, out.strides[0], rb, rb, re, scratch.ctypes.data,
                                 scratch.nbytes, LUT.ctypes.data, quality=quality)
     rc = lib.emu_develop(C.byref(a), tile[0], tile[1])
