@@ -59,6 +59,19 @@ extern "C" {
  * or displays the image needs, at 3 / 6 instead of 12 bytes per pixel over PCIe. */
 #define PYSP_OUT_SRGB_U8 3
 #define PYSP_OUT_SRGB_U16 4
+/* JPEG-ready planes, 1.5 bytes per pixel: the PYSP_OUT_SRGB_U8 result S[y][x][0..2] = R, G, B of the same call, converted
+ * exactly as libjpeg converts and subsamples it for a 4:2:0 JPEG (jccolor.c rgb_ycc_convert, full-range JFIF / BT.601;
+ * jcsample.c h2v2_downsample), so that a JPEG encoded from the planes is byte-identical to one libjpeg encodes from S.
+ * Integer arithmetic, arithmetic shifts, stored orientation:
+ *     Y [y][x]   = (19595*R + 38470*G + 7471*B + 32768) >> 16
+ *     cb[y][x]   = (-11059*R - 21709*G + 32768*B + (128 << 16) + 32767) >> 16
+ *     cr[y][x]   = (32768*R - 27439*G - 5329*B + (128 << 16) + 32767) >> 16
+ *     Cb[cy][cx] = (cb[2cy][2cx] + cb[2cy][2cx+1] + cb[2cy+1][2cx] + cb[2cy+1][2cx+1] + 1 + (cx & 1)) >> 2   (Cr alike)
+ * cx is the chroma column of the whole stored frame.  `out` holds Y ([rows][width], pitch out_pitch_bytes >= width),
+ * `out_cb` / `out_cr` hold Cb / Cr ([rows/2][width/2], pitch out_chroma_pitch_bytes >= width/2).  Y row 0 is stored row
+ * out_row0 (which must be even), chroma row 0 is stored chroma row out_row0/2; a band [row_begin, row_end) writes Y rows
+ * [row_begin, row_end) and chroma rows [row_begin/2, row_end/2) only. */
+#define PYSP_OUT_YCC420_U8 5
 
 /* const.py:3-6 (QualityDemosaic); Draft is not on the B200 path */
 #define PYSP_QUALITY_BEST 0
@@ -88,7 +101,8 @@ typedef struct pysp_develop_args {
     int32_t is_hdr;              /* image.get_hdr() (debayer/ahd.py:52-59) */
     int32_t apply_gamma;         /* fuse lin_srgb_to_srgb (colorize/transform.py:89-99) into the epilogue */
     int32_t out_kind;            /* PYSP_OUT_* */
-    void* out;                   /* [rows][width][3], rows [out_row0, ...) of the frame as stored */
+    void* out;                   /* [rows][width][3], rows [out_row0, ...) of the frame as stored (Y plane
+                                    [rows][width] for PYSP_OUT_YCC420_U8) */
     int64_t out_pitch_bytes;
     int32_t out_row0;
     int32_t row_begin, row_end;  /* stored rows to produce, even; whole frame = [0, height) */
@@ -102,6 +116,11 @@ typedef struct pysp_develop_args {
                                     [rows][width] for rows [out_row0, ...) of the frame as stored.  The reference never
                                     returns this map; it is exported so that parity of the choice can be checked. */
     int64_t dir_map_pitch_bytes;
+    /* PYSP_OUT_YCC420_U8 only (appended: the library reads these three fields for that kind alone, so callers built
+       against the struct without them stay valid for every other kind) */
+    void* out_cb;                /* [rows/2][width/2] Cb, chroma rows [out_row0/2, ...) of the frame as stored */
+    void* out_cr;                /* [rows/2][width/2] Cr, same rows */
+    int64_t out_chroma_pitch_bytes;
 } pysp_develop_args;
 
 int pysp_develop(const pysp_develop_args* args, void* stream);

@@ -12,7 +12,7 @@ LIB_PATH = os.environ.get("PYSP_B200_LIB") or os.path.join(_HERE, "libpysp_b200.
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA = 0, -1, -2, -3
 CFA = {"RGGB": 1, "BGGR": 2, "GRBG": 3, "GBRG": 4}
 IN_U16, IN_F32 = 0, 1
-OUT_CAM_F32, OUT_LIN_F32, OUT_LIN_F16, OUT_SRGB_U8, OUT_SRGB_U16 = 0, 1, 2, 3, 4
+OUT_CAM_F32, OUT_LIN_F32, OUT_LIN_F16, OUT_SRGB_U8, OUT_SRGB_U16, OUT_YCC420_U8 = 0, 1, 2, 3, 4, 5
 QUALITY_BEST, QUALITY_FAST = 0, 1
 MAX_BRACKETS = 16
 
@@ -33,6 +33,7 @@ class DevelopArgs(C.Structure):
         ("lab_lut", C.c_void_p),
         ("quality", C.c_int32),
         ("dir_map", C.c_void_p), ("dir_map_pitch_bytes", C.c_int64),
+        ("out_cb", C.c_void_p), ("out_cr", C.c_void_p), ("out_chroma_pitch_bytes", C.c_int64),
     ]
 
 
@@ -126,7 +127,8 @@ def check(rc, last_error=None):
 
 def fill_develop_args(height, width, pattern, in_kind, in_ptr, in_pitch, in_row0, in_rows, black, white, wb,
                       cam_to_srgb, stages, is_hdr, gamma, out_kind, out_ptr, out_pitch, out_row0, row_begin,
-                      row_end, scratch_ptr, scratch_bytes, lut_ptr, quality=0, dir_map_ptr=None, dir_map_pitch=0):
+                      row_end, scratch_ptr, scratch_bytes, lut_ptr, quality=0, dir_map_ptr=None, dir_map_pitch=0,
+                      out_cb_ptr=None, out_cr_ptr=None, out_chroma_pitch=0):
     a = DevelopArgs()
     a.height, a.width = int(height), int(width)
     if isinstance(pattern, str):
@@ -160,4 +162,6 @@ def fill_develop_args(height, width, pattern, in_kind, in_ptr, in_pitch, in_row0
     a.quality = int(quality)
     a.dir_map = dir_map_ptr
     a.dir_map_pitch_bytes = int(dir_map_pitch)
+    a.out_cb, a.out_cr = out_cb_ptr, out_cr_ptr
+    a.out_chroma_pitch_bytes = int(out_chroma_pitch)
     return a

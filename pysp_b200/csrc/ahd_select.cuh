@@ -123,7 +123,56 @@ PYSP_HD void store_tile_generic(const float* out, const StoreParams& st, const F
     int bx, by;
     tile_output_box<TW, TH>(st, g, x0, y0, &bx, &by);
     if (st.mode == OUT_FINAL) {
-        if (st.kind == OUT_LIN_F16 || st.kind >= OUT_SRGB_U8) {
+        if (st.kind == OUT_YCC420_U8) {
+            // JPEG-ready planes: quantise like OUT_SRGB_U8, then libjpeg's integer YCbCr and 4:2:0 average (ycc_block).  A work
+            // item is a 2x2 block of the staging tile (2x4 on the word path).  Blocks are 2-aligned in stored coordinates:
+            // tile origins, W, H and band bounds are even, also under a flip (the stored origin W - (x0 + TW) is even), so a
+            // block lies wholly inside the destination or wholly outside it (partial tiles, negative origins of flipped
+            // partial tiles): outside blocks are skipped.  The chroma bias alternates along the STORED chroma column.
+            const int sx = bx / 3;                                    // stored column of the tile's first pixel (even)
+            auto block = [&](int r, int c, uint32_t bias) {           // staging row r, column c (both even)
+                uint32_t R[4], G[4], B[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const float* p = out + (r + (k >> 1)) * (TW * 3) + (c + (k & 1)) * 3;
+                    R[k] = quantise(p[0], 255.0f); G[k] = quantise(p[1], 255.0f); B[k] = quantise(p[2], 255.0f);
+                }
+                return ycc_block(R, G, B, bias);
+            };
+            char* const yb = (char*)st.img.base;
+            char* const cbb = (char*)st.cb.base;
+            char* const crb = (char*)st.cr.base;
+            const bool words = by >= 0 && by + TH <= st.img.rows && sx >= 0 && sx + TW <= st.img.cols && (sx & 3) == 0 &&
+                               st.img.pitch % 4 == 0 && ((uintptr_t)yb % 4) == 0 && st.cb.pitch % 2 == 0 && st.cr.pitch % 2 == 0 &&
+                               ((uintptr_t)cbb % 2) == 0 && ((uintptr_t)crb % 2) == 0;
+            static_assert(TW % 4 == 0 && TH % 2 == 0, "a tile is a whole number of 2x4 blocks");
+            if (words) {
+                // 2x4 block: two 32-bit Y words and one 16-bit word per chroma plane; its left chroma column is even
+                constexpr int BPR = TW / 4;
+                PYSP_ITEMS(i, (TH / 2) * BPR) {
+                    const int j = i / BPR, c = 4 * (i - j * BPR), y = by + 2 * j, cy = y >> 1, cx = (sx + c) >> 1;
+                    const Ycc2x2 a = block(2 * j, c, 1u), b = block(2 * j, c + 2, 2u);
+                    *(uint32_t*)(yb + (long long)y * st.img.pitch + sx + c) = a.y01 | (b.y01 << 16);
+                    *(uint32_t*)(yb + (long long)(y + 1) * st.img.pitch + sx + c) = a.y23 | (b.y23 << 16);
+                    *(uint16_t*)(cbb + (long long)cy * st.cb.pitch + cx) = (uint16_t)(a.cb | (b.cb << 8));
+                    *(uint16_t*)(crb + (long long)cy * st.cr.pitch + cx) = (uint16_t)(a.cr | (b.cr << 8));
+                }
+            } else {
+                constexpr int BPR = TW / 2;
+                PYSP_ITEMS(i, (TH / 2) * BPR) {
+                    const int j = i / BPR, c = 2 * (i - j * BPR), y = by + 2 * j, x = sx + c;
+                    if (y < 0 || y >= st.img.rows || x < 0 || x >= st.img.cols) continue;
+                    const int cy = y >> 1, cx = x >> 1;
+                    const Ycc2x2 a = block(2 * j, c, 1u + (cx & 1));
+                    uint8_t* y0p = (uint8_t*)(yb + (long long)y * st.img.pitch + x);
+                    uint8_t* y1p = (uint8_t*)(yb + (long long)(y + 1) * st.img.pitch + x);
+                    y0p[0] = (uint8_t)a.y01; y0p[1] = (uint8_t)(a.y01 >> 8);
+                    y1p[0] = (uint8_t)a.y23; y1p[1] = (uint8_t)(a.y23 >> 8);
+                    ((uint8_t*)(cbb + (long long)cy * st.cb.pitch))[cx] = (uint8_t)a.cb;
+                    ((uint8_t*)(crb + (long long)cy * st.cr.pitch))[cx] = (uint8_t)a.cr;
+                }
+            }
+        } else if (st.kind == OUT_LIN_F16 || st.kind >= OUT_SRGB_U8) {
             // narrow outputs: converted on the way out of the float staging tile (consecutive threads write consecutive
             // elements of a tile row).  Quantised sRGB: round-to-nearest of the gamma-encoded value times 255 / 65535.
             // A tile that lies inside the image with 4-byte aligned rows leaves as packed 32-bit words (four u8 or two

@@ -89,7 +89,7 @@ static inline int plan_develop(const pysp_develop_args* a, int tw1, int th1, int
     }
     if (a->in_kind != PYSP_IN_U16 && a->in_kind != PYSP_IN_F32)
         return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: bad in_kind %d", a->in_kind);
-    if (a->out_kind < PYSP_OUT_CAM_F32 || a->out_kind > PYSP_OUT_SRGB_U16)
+    if (a->out_kind < PYSP_OUT_CAM_F32 || a->out_kind > PYSP_OUT_YCC420_U8)
         return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: bad out_kind %d", a->out_kind);
     if (!a->in || !a->out || (!a->lab_lut && a->quality == PYSP_QUALITY_BEST))
         return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: null buffer");
@@ -108,8 +108,19 @@ static inline int plan_develop(const pysp_develop_args* a, int tw1, int th1, int
     if (a->in_pitch_bytes < W * esz || (a->in_pitch_bytes % esz) || ((uintptr_t)a->in % esz))
         return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: bad input pitch/alignment");
     const int64_t osz = out_kind_bytes(a->out_kind);
-    if (a->out_pitch_bytes < 3 * W * osz || (a->out_pitch_bytes % osz) || ((uintptr_t)a->out % osz))
+    const bool ycc = a->out_kind == PYSP_OUT_YCC420_U8;
+    const int out_cols = ycc ? W : 3 * W;                 // elements of an output row (YCbCr 4:2:0: of the Y plane)
+    if (a->out_pitch_bytes < out_cols * osz || (a->out_pitch_bytes % osz) || ((uintptr_t)a->out % osz))
         return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: bad output pitch/alignment");
+    if (ycc) {                                            // the chroma fields are read for this kind only
+        if (!a->out_cb || !a->out_cr)
+            return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: null Cb or Cr plane");
+        if (a->out_chroma_pitch_bytes < W / 2)
+            return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: chroma pitch %lld is shorter than W/2 = %d",
+                             (long long)a->out_chroma_pitch_bytes, W / 2);
+        if (a->out_row0 & 1)
+            return plan_fail(err, errn, PYSP_ERR_INVALID, "pysp_develop: out_row0 %d must be even for 4:2:0 output", a->out_row0);
+    }
     // logical (RGGB-oriented) rows of the band
     const int lb = flip_y ? H - re : rb, le = flip_y ? H - rb : re;
     auto lo = [&](int v) { return v < 0 ? 0 : v; };
@@ -139,8 +150,14 @@ static inline int plan_develop(const pysp_develop_args* a, int tw1, int th1, int
     auto final_store = [&](StoreParams& st) {
         st.mode = OUT_FINAL; st.kind = a->out_kind;
         st.img.base = (char*)a->out + (int64_t)(rb - a->out_row0) * a->out_pitch_bytes;
-        st.img.pitch = a->out_pitch_bytes; st.img.rows = re - rb; st.img.cols = 3 * W; st.img.elem = (int)osz;
+        st.img.pitch = a->out_pitch_bytes; st.img.rows = re - rb; st.img.cols = out_cols; st.img.elem = (int)osz;
         st.img_row0 = rb;
+        if (ycc) {
+            const int64_t c0 = (int64_t)(rb - a->out_row0) / 2 * a->out_chroma_pitch_bytes;   // chroma row rb/2 of the views
+            st.cb.base = (char*)a->out_cb + c0; st.cr.base = (char*)a->out_cr + c0;
+            st.cb.pitch = st.cr.pitch = a->out_chroma_pitch_bytes;
+            st.cb.rows = st.cr.rows = (re - rb) / 2; st.cb.cols = st.cr.cols = W / 2; st.cb.elem = st.cr.elem = 1;
+        }
         st.tma = osz == 4 && tma_ok(st.img, flip_x != 0, (long long)W * 12);
     };
     auto plane_store = [&](StoreParams& st, int buf, int row0, int rows) {

@@ -73,13 +73,16 @@ namespace pysp {
 #define PYSP_GK1 (0.45186275f)
 
 enum InKind { IN_U16 = 0, IN_F32 = 1 };
-enum OutKind { OUT_CAM_F32 = 0, OUT_LIN_F32 = 1, OUT_LIN_F16 = 2, OUT_SRGB_U8 = 3, OUT_SRGB_U16 = 4 };
+enum OutKind { OUT_CAM_F32 = 0, OUT_LIN_F32 = 1, OUT_LIN_F16 = 2, OUT_SRGB_U8 = 3, OUT_SRGB_U16 = 4, OUT_YCC420_U8 = 5 };
 #ifdef __CUDACC__
 #define PYSP_HOSTDEV __host__ __device__
 #else
 #define PYSP_HOSTDEV
 #endif
-PYSP_HOSTDEV constexpr int out_kind_bytes(int kind) { return kind == OUT_SRGB_U8 ? 1 : ((kind == OUT_LIN_F16 || kind == OUT_SRGB_U16) ? 2 : 4); }
+// bytes per stored element (for OUT_YCC420_U8: per sample of any of its three planes)
+PYSP_HOSTDEV constexpr int out_kind_bytes(int kind) {
+    return (kind == OUT_SRGB_U8 || kind == OUT_YCC420_U8) ? 1 : ((kind == OUT_LIN_F16 || kind == OUT_SRGB_U16) ? 2 : 4);
+}
 
 struct FrameGeom {
     int H, W;            // frame size (even); flips keep the size
@@ -111,6 +114,8 @@ struct StoreParams {
     int mode;            // OutMode
     int kind;            // OutKind (final only)
     View2D img;          // final: [band rows][3*W] of f32/f16; row 0 = first stored row of the band
+                         //   (OUT_YCC420_U8: the Y plane, [band rows][W])
+    View2D cb, cr;       // OUT_YCC420_U8 only: [band rows / 2][W / 2]; row 0 = stored chroma row img_row0 / 2
     int img_row0;        // stored row number of img row 0
     View2D plane[3];     // planes: [rows][W] f32, row 0 = logical row plane_row0
     int plane_row0;
@@ -207,6 +212,26 @@ PYSP_HD float srgb_gamma(float v) {
 PYSP_HD uint32_t quantise(float v, float scale) {
     float y = fmaf(sat01(v), scale, 8388608.0f);        // v * scale <= 65535 is below 2^23: adding 2^23 rounds to an integer
     return pysp_as_uint(y) & 0x7FFFFFu;
+}
+
+// libjpeg's full-range R'G'B' -> YCbCr (jccolor.c rgb_ycc_convert, 16-bit fixed point) and 2x2 chroma average
+// (jcsample.c h2v2_downsample) of one 2x2 block of 8-bit pixels.  r[k], g[k], b[k]: pixels TL, TR, BL, BR.  bias: 1 for an
+// even stored chroma column, 2 for an odd one.  y01 / y23: the block's top / bottom Y pair, left pixel in the low byte.
+// Every intermediate is non-negative (the chroma offset (128 << 16) + 32767 exceeds 0.5 * 255 * 65536), so the shifts
+// are the arithmetic shifts of the C source.
+struct Ycc2x2 { uint32_t y01, y23, cb, cr; };
+PYSP_HD Ycc2x2 ycc_block(const uint32_t r[4], const uint32_t g[4], const uint32_t b[4], uint32_t bias) {
+    Ycc2x2 o;
+    uint32_t y[4], cb = 0, cr = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        y[k] = (19595u * r[k] + 38470u * g[k] + 7471u * b[k] + 32768u) >> 16;
+        cb += (32768u * b[k] + (128u << 16) + 32767u - 11059u * r[k] - 21709u * g[k]) >> 16;
+        cr += (32768u * r[k] + (128u << 16) + 32767u - 27439u * g[k] - 5329u * b[k]) >> 16;
+    }
+    o.y01 = y[0] | (y[1] << 8); o.y23 = y[2] | (y[3] << 8);
+    o.cb = (cb + bias) >> 2; o.cr = (cr + bias) >> 2;
+    return o;
 }
 
 // ---- cv2 RGB->Lab (float32 path) : quantise, trilinear in the 33^3 int16 table -----------------------

@@ -116,9 +116,38 @@ def to_device(a, device=None, dtype=None, pad_pitch=False):
 
 
 _OUT_KINDS = {"cam": _capi.OUT_CAM_F32, "lin": _capi.OUT_LIN_F32, "lin_f16": _capi.OUT_LIN_F16,
-              "srgb_u8": _capi.OUT_SRGB_U8, "srgb_u16": _capi.OUT_SRGB_U16}
+              "srgb_u8": _capi.OUT_SRGB_U8, "srgb_u16": _capi.OUT_SRGB_U16, "ycc420": _capi.OUT_YCC420_U8}
 _OUT_DTYPES = {_capi.OUT_CAM_F32: torch.float32, _capi.OUT_LIN_F32: torch.float32, _capi.OUT_LIN_F16: torch.float16,
-               _capi.OUT_SRGB_U8: torch.uint8, _capi.OUT_SRGB_U16: torch.uint16}
+               _capi.OUT_SRGB_U8: torch.uint8, _capi.OUT_SRGB_U16: torch.uint16, _capi.OUT_YCC420_U8: torch.uint8}
+
+
+def i420_bytes(rows, width):
+    """bytes of one I420 buffer (Y [rows, W], then Cb and Cr [rows/2, W/2]) of an even-sized image"""
+    return int(rows) * int(width) * 3 // 2
+
+
+def i420_planes(buf, rows, width):
+    """(y, cb, cr): uint8 views [rows, W], [rows/2, W/2], [rows/2, W/2] over the first i420_bytes(rows, W) bytes of the flat
+    uint8 tensor `buf`, Y first, then Cb, then Cr -- the layout a JPEG encoder's raw-data input takes, moved by one copy."""
+    rows, width = int(rows), int(width)
+    if rows % 2 or width % 2 or buf.dtype != torch.uint8 or buf.dim() != 1 or buf.numel() < i420_bytes(rows, width):
+        raise ValueError("i420_planes: a flat uint8 buffer of >= %d bytes and an even size are needed" % i420_bytes(rows, width))
+    ny, nc = rows * width, (rows // 2) * (width // 2)
+    return (buf[:ny].view(rows, width), buf[ny:ny + nc].view(rows // 2, width // 2),
+            buf[ny + nc:ny + 2 * nc].view(rows // 2, width // 2))
+
+
+def _check_ycc_planes(planes, rows, W):
+    ok = isinstance(planes, (tuple, list)) and len(planes) == 3
+    if ok:
+        y, cb, cr = planes
+        ok = all(t.is_cuda and t.dtype == torch.uint8 and t.dim() == 2 and t.stride(1) == 1 for t in planes) and \
+            y.shape[1] == W and y.shape[0] >= rows and cb.stride(0) == cr.stride(0) and \
+            all(t.shape[1] == W // 2 and t.shape[0] >= rows // 2 for t in (cb, cr))
+    if not ok:
+        raise ValueError("engine.develop: out_tensor for out='ycc420' must be (y, cb, cr) uint8 CUDA views [rows, W], "
+                         "[rows/2, W/2], [rows/2, W/2] with unit column stride and one chroma pitch")
+    return planes
 
 
 def develop(mosaic, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white=None, hdr=False, gamma=False,
@@ -133,8 +162,11 @@ def develop(mosaic, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white
     quality     "best" = AHD (debayer_ahd), "fast" = edge-assisted Gaussian (debayer_eag; stages/hdr ignored).
     dir_map     optional CUDA uint8 tensor [>= row_end-out_row0, W]: receives the AHD direction choice (1 = horizontal).
     out         "cam" (camera RGB), "lin" (linear sRGB, float32), "lin_f16", or the wire formats "srgb_u8" / "srgb_u16"
-                (lin_srgb_to_srgb, then rounded into 8 / 16 bits).
-    Returns a CUDA tensor [row_end-row_begin, W, 3] of the matching dtype.
+                (lin_srgb_to_srgb, then rounded into 8 / 16 bits) and "ycc420": the srgb_u8 result as libjpeg converts and
+                subsamples it for a 4:2:0 JPEG (full-range YCbCr; include/pysp_b200.h, PYSP_OUT_YCC420_U8).
+    Returns a CUDA tensor [row_end-row_begin, W, 3] of the matching dtype; for "ycc420" the uint8 planes (y, cb, cr) of
+    shapes [n, W], [n/2, W/2], [n/2, W/2] (n = row_end - out_row0) over ONE contiguous I420 buffer (i420_planes), or
+    `out_tensor` itself, which is then such a triple with any row pitches (Cb and Cr sharing one).
     """
     if quality not in ("best", "fast"):
         raise NotImplementedError("Quality mode not implemented: %s" % str(quality))
@@ -165,10 +197,17 @@ def develop(mosaic, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white
     if dir_map is not None and (not dir_map.is_cuda or dir_map.dtype != torch.uint8 or dir_map.dim() != 2
                                 or dir_map.shape[1] != W or dir_map.stride(1) != 1 or dir_map.shape[0] < re - out_row0):
         raise ValueError("engine.develop: dir_map must be a CUDA uint8 tensor [rows, W]")
+    ycc = kind == _capi.OUT_YCC420_U8
     with _on(dev, stream):
         if mosaic.stride(1) != 1:
             mosaic = mosaic.contiguous()
-        if out_tensor is None:
+        if ycc:
+            if out_tensor is None:
+                n = re - out_row0
+                out_tensor = i420_planes(torch.empty(i420_bytes(n, W), dtype=torch.uint8, device=dev), n, W)
+            else:
+                out_tensor = _check_ycc_planes(out_tensor, re - out_row0, W)
+        elif out_tensor is None:
             out_tensor = torch.empty((re - out_row0, W, 3), dtype=odt, device=dev)
         elif (not out_tensor.is_cuda or out_tensor.dtype != odt or out_tensor.dim() != 3
               or out_tensor.shape[1] != W or out_tensor.shape[2] != 3 or out_tensor.stride(2) != 1
@@ -177,14 +216,17 @@ def develop(mosaic, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white
         nscr = int(L.pysp_develop_scratch_bytes(W, re - rb, int(stages)))
         scratch = _get_scratch(dev, nscr, stream)
         lut = lab_lut(dev)
+        dst = out_tensor[0] if ycc else out_tensor
         a = _capi.fill_develop_args(
             H, W, pattern, in_kind, mosaic.data_ptr(), mosaic.stride(0) * mosaic.element_size(), in_row0, held,
-            black, white, wb, cam_to_srgb, stages, hdr, gamma, kind, out_tensor.data_ptr(),
-            out_tensor.stride(0) * out_tensor.element_size(), out_row0, rb, re,
+            black, white, wb, cam_to_srgb, stages, hdr, gamma, kind, dst.data_ptr(),
+            dst.stride(0) * dst.element_size(), out_row0, rb, re,
             scratch.data_ptr() if scratch is not None else None, nscr, lut.data_ptr(),
             quality=_capi.QUALITY_FAST if quality == "fast" else _capi.QUALITY_BEST,
             dir_map_ptr=dir_map.data_ptr() if dir_map is not None else None,
-            dir_map_pitch=dir_map.stride(0) if dir_map is not None else 0)
+            dir_map_pitch=dir_map.stride(0) if dir_map is not None else 0,
+            out_cb_ptr=out_tensor[1].data_ptr() if ycc else None, out_cr_ptr=out_tensor[2].data_ptr() if ycc else None,
+            out_chroma_pitch=out_tensor[1].stride(0) if ycc else 0)
         _capi.check(L.pysp_develop(C.byref(a), _stream_ptr(stream)))
     return out_tensor
 
