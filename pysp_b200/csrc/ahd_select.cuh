@@ -296,6 +296,79 @@ PYSP_HD void up_br(const float v[3][3], float o[4]) {
 
 PYSP_HD float gauss_row(float l, float c, float r) { return (PYSP_GK1 * c) + (PYSP_GK0 * (l + r)); }
 
+// The resample step both demosaics share (edge_assisted_gaussian.py:126-143; AHD runs it per direction, ahd.py:120-127):
+// 3x3 Gaussian high-pass of the full-resolution green, 4-phase Gaussian upsample of c - g and g, and their sums, for the
+// quad at local quarter index (i, j) of a tile whose quarter planes start at frame quarter index (qy0, qx0).
+// GR / GB: green at R / B sites, DR / DB: R - g / B - g, G1 / G2: the balanced native greens.  v gets TL, TR, BL, BR.
+template <int TW, int TH, bool EDGE>
+PYSP_HD void quad_resample(const float* GR, const float* GB, const float* DR, const float* DB, const float* G1,
+                           const float* G2, int i, int j, int qy0, int qx0, int H, int W, Rgb v[4]) {
+    constexpr int QW = SelectTile<TW, TH>::QW;
+    const int fi = qy0 + i, fj = qx0 + j;              // frame quarter index
+    // local quarter row/col of the 3 neighbours under quarter-grid REFLECT_101
+    int ri[3], cj[3];
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        ri[d] = EDGE ? reflect101(fi + d - 1, H >> 1) - qy0 : i + d - 1;
+        cj[d] = EDGE ? reflect101(fj + d - 1, W >> 1) - qx0 : j + d - 1;
+    }
+    float gr[3][3], gb[3][3], dr[3][3], db[3][3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) {
+            int c = ri[a] * QW + cj[b];
+            gr[a][b] = GR[c]; gb[a][b] = GB[c]; dr[a][b] = DR[c]; db[a][b] = DB[c];
+        }
+    // full-res green window rows 2i-1..2i+2, cols 2j-1..2j+2 for the high-pass, with full-res REFLECT_101
+    // (ahd.py:120).  Reflection keeps the CFA phase, so the plane of every window cell is static; only its quarter
+    // index moves at the frame border.
+    float gw[4][4];
+    {
+        int wr[4], wc[4];
+        if (EDGE) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                wr[k] = (reflect101(2 * fi - 1 + k, H) >> 1) - qy0;
+                wc[k] = (reflect101(2 * fj - 1 + k, W) >> 1) - qx0;
+            }
+        } else {
+            wr[0] = i - 1; wr[1] = i; wr[2] = i; wr[3] = i + 1;
+            wc[0] = j - 1; wc[1] = j; wc[2] = j; wc[3] = j + 1;
+        }
+#pragma unroll
+        for (int a = 0; a < 4; ++a)
+#pragma unroll
+            for (int b = 0; b < 4; ++b) {
+                int c = wr[a] * QW + wc[b];
+                const bool oddrow = (a & 1) == 0, oddcol = (b & 1) == 0;   // window starts at -1
+                gw[a][b] = oddrow ? (oddcol ? GB[c] : G2[c]) : (oddcol ? G1[c] : GR[c]);
+            }
+    }
+    float hf[4];
+    {
+        float rp[4][2];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) {
+            rp[a][0] = gauss_row(gw[a][0], gw[a][1], gw[a][2]);
+            rp[a][1] = gauss_row(gw[a][1], gw[a][2], gw[a][3]);
+        }
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int b = 0; b < 2; ++b)
+                hf[a * 2 + b] = gw[a + 1][b + 1] - gauss_row(rp[a][b], rp[a + 1][b], rp[a + 2][b]);
+    }
+    float ugr[4], udr[4], ugb[4], udb[4];
+    up_tl(gr, ugr); up_tl(dr, udr); up_br(gb, ugb); up_br(db, udb);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        v[k].r = udr[k] + (ugr[k] + hf[k]);          // edge_assisted_gaussian.py:141-143
+        v[k].b = udb[k] + (ugb[k] + hf[k]);
+        v[k].g = gw[1 + (k >> 1)][1 + (k & 1)];
+    }
+}
+
 // ---- phase 0: staging box -> normalised, white-balanced quarter planes -------------------------------------
 // normalization.py:20-23 on one photosite: clip(raw - black, 0, white) / white.  The IEEE division is replaced,
 // when the host has checked it exhaustively for these levels (all 65536 sensor codes, develop_plan.h), by the
@@ -421,78 +494,13 @@ PYSP_D void select_phases(const SelectParams& p, char* __restrict__ smem, int ti
             int i = py + IY - 1, j = px + JX - 1;      // local quarter index
             int fi = qy0 + i, fj = qx0 + j;            // frame quarter index
             if (EDGE) { if (fi < 0 || fi >= hq || fj < 0 || fj >= wq || 2 * fi >= p.y_end + 2) continue; }
-            // local quarter row/col of the 3 neighbours under quarter-grid REFLECT_101
-            int ri[3], cj[3];
-#pragma unroll
-            for (int d = 0; d < 3; ++d) {
-                ri[d] = EDGE ? reflect101(fi + d - 1, hq) - qy0 : i + d - 1;
-                cj[d] = EDGE ? reflect101(fj + d - 1, wq) - qx0 : j + d - 1;
-            }
             const bool inner = py >= 1 && py <= TH / 2 && px >= 1 && px <= TW / 2;
 #pragma unroll 1                                       // one copy of the body (measured: unrolling both directions is 2 % slower)
             for (int dir = 0; dir < 2; ++dir) {
-                const float* GR = Q + (dir ? L::P_GVR : L::P_GHR) * QN;
-                const float* GB = Q + (dir ? L::P_GVB : L::P_GHB) * QN;
-                const float* DR = Q + (dir ? L::P_DVR : L::P_DHR) * QN;
-                const float* DB = Q + (dir ? L::P_DVB : L::P_DHB) * QN;
-                const float* G1 = Q + L::P_G1 * QN;
-                const float* G2 = Q + L::P_G2 * QN;
-                float gr[3][3], gb[3][3], dr[3][3], db[3][3];
-#pragma unroll
-                for (int a = 0; a < 3; ++a)
-#pragma unroll
-                    for (int b = 0; b < 3; ++b) {
-                        int c = ri[a] * QW + cj[b];
-                        gr[a][b] = GR[c]; gb[a][b] = GB[c]; dr[a][b] = DR[c]; db[a][b] = DB[c];
-                    }
-                // full-res green window rows 2i-1..2i+2, cols 2j-1..2j+2 for the high-pass, with full-res
-                // REFLECT_101 (ahd.py:120).  Reflection keeps the CFA phase, so the plane of every window
-                // cell is static; only its quarter index moves at the frame border.
-                float gw[4][4];
-                {
-                    int wr[4], wc[4];
-                    if (EDGE) {
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            wr[k] = (reflect101(2 * fi - 1 + k, H) >> 1) - qy0;
-                            wc[k] = (reflect101(2 * fj - 1 + k, W) >> 1) - qx0;
-                        }
-                    } else {
-                        wr[0] = i - 1; wr[1] = i; wr[2] = i; wr[3] = i + 1;
-                        wc[0] = j - 1; wc[1] = j; wc[2] = j; wc[3] = j + 1;
-                    }
-#pragma unroll
-                    for (int a = 0; a < 4; ++a)
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) {
-                            int c = wr[a] * QW + wc[b];
-                            const bool oddrow = (a & 1) == 0, oddcol = (b & 1) == 0;   // window starts at -1
-                            gw[a][b] = oddrow ? (oddcol ? GB[c] : G2[c]) : (oddcol ? G1[c] : GR[c]);
-                        }
-                }
-                float hf[4];
-                {
-                    float rp[4][2];
-#pragma unroll
-                    for (int a = 0; a < 4; ++a) {
-                        rp[a][0] = gauss_row(gw[a][0], gw[a][1], gw[a][2]);
-                        rp[a][1] = gauss_row(gw[a][1], gw[a][2], gw[a][3]);
-                    }
-#pragma unroll
-                    for (int a = 0; a < 2; ++a)
-#pragma unroll
-                        for (int b = 0; b < 2; ++b)
-                            hf[a * 2 + b] = gw[a + 1][b + 1] - gauss_row(rp[a][b], rp[a + 1][b], rp[a + 2][b]);
-                }
-                float ugr[4], udr[4], ugb[4], udb[4];
-                up_tl(gr, ugr); up_tl(dr, udr); up_br(gb, ugb); up_br(db, udb);
-                float Rc[4], Gc[4], Bc[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    Rc[k] = udr[k] + (ugr[k] + hf[k]);          // edge_assisted_gaussian.py:141-143
-                    Bc[k] = udb[k] + (ugb[k] + hf[k]);
-                    Gc[k] = gw[1 + (k >> 1)][1 + (k & 1)];
-                }
+                Rgb cv[4];                             // this direction's candidate pixels TL, TR, BL, BR
+                quad_resample<TW, TH, EDGE>(Q + (dir ? L::P_GVR : L::P_GHR) * QN, Q + (dir ? L::P_GVB : L::P_GHB) * QN,
+                                            Q + (dir ? L::P_DVR : L::P_DHR) * QN, Q + (dir ? L::P_DVB : L::P_DHB) * QN,
+                                            Q + L::P_G1 * QN, Q + L::P_G2 * QN, i, j, qy0, qx0, H, W, cv);
                 // Lab of the metric image, kept for the tile + 2 px
                 float* oL = labL + dir * (L::LH * L::LW);
                 uint32_t* oAB = labAB + dir * (L::LH * L::LW);
@@ -503,14 +511,14 @@ PYSP_D void select_phases(const SelectParams& p, char* __restrict__ smem, int ti
                     float m3[3], luma[4];
                     LabKey key[2];
                     uint4 e[2][4];
-                    metric_rgb(p.c, Rc[0], Gc[0], Bc[0], m3, &luma[0]);
+                    metric_rgb(p.c, cv[0].r, cv[0].g, cv[0].b, m3, &luma[0]);
                     key[0] = lab_key(p.lut, m3[0], m3[1], m3[2]);
 #pragma unroll
                     for (int c = 0; c < 4; ++c) e[0][c] = pysp_ldg(key[0].base + (c >> 1) * PYSP_LUT_NG * PYSP_LUT_NB + (c & 1) * PYSP_LUT_NB);
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         if (k < 3) {
-                            metric_rgb(p.c, Rc[k + 1], Gc[k + 1], Bc[k + 1], m3, &luma[k + 1]);
+                            metric_rgb(p.c, cv[k + 1].r, cv[k + 1].g, cv[k + 1].b, m3, &luma[k + 1]);
                             key[(k + 1) & 1] = lab_key(p.lut, m3[0], m3[1], m3[2]);
 #pragma unroll
                             for (int c = 0; c < 4; ++c)
@@ -535,8 +543,8 @@ PYSP_D void select_phases(const SelectParams& p, char* __restrict__ smem, int ti
 #pragma unroll
                     for (int a = 0; a < 2; ++a) {
                         const int o = (2 * (py - 1) + a) * TW + 2 * (px - 1);
-                        F2 r2; r2.x = Rc[2 * a]; r2.y = Rc[2 * a + 1];
-                        F2 b2; b2.x = Bc[2 * a]; b2.y = Bc[2 * a + 1];
+                        F2 r2; r2.x = cv[2 * a].r; r2.y = cv[2 * a + 1].r;
+                        F2 b2; b2.x = cv[2 * a].b; b2.y = cv[2 * a + 1].b;
                         *(F2*)(oR + o) = r2; *(F2*)(oB + o) = b2;
                     }
                 }

@@ -2,7 +2,8 @@
 // tile pipeline as K1.  Phase 0 (ahd_select.cuh) leaves the greens un-balanced here, because the reference
 // interpolates the raw greens and multiplies by wb[1] afterwards (edge_assisted_gaussian.py:193).
 //   phase 1  green at R/B sites by the delta-mix bilinear kernel (l.10-49, 92-124), white balance, colour differences;
-//   phase 2  per 2x2 quad: green high-pass (l.157), 4-phase Gaussian upsample of (c-g) and g (l.126-143) -> staging tile.
+//   phase 2  per 2x2 quad: green high-pass (l.157), 4-phase Gaussian upsample of (c-g) and g (l.126-143) -> staging tile,
+//            by K1's quad_resample.
 #pragma once
 #include "ahd_select.cuh"
 
@@ -55,68 +56,16 @@ PYSP_D void eag_phases(const SelectParams& p, char* __restrict__ smem, int tile_
     PYSP_SYNC();
     {
         constexpr int OW = TW / 2, OH = TH / 2;
-        const float* GR = Q + L::P_GHR * QN; const float* GB = Q + L::P_GHB * QN;
-        const float* G1 = Q + L::P_GVR * QN; const float* G2 = Q + L::P_GVB * QN;
-        const float* DR = Q + L::P_DHR * QN; const float* DB = Q + L::P_DHB * QN;
         PYSP_ITEMS(it, OW * OH) {
             int oy = it / OW, ox = it - oy * OW;
             int i = oy + IY, j = ox + JX;
             int fi = qy0 + i, fj = qx0 + j;
             if (EDGE) { if (fi >= hq || fj >= wq || 2 * fi >= p.y_end) continue; }
-            int ri[3], cj[3];
+            Rgb v[4];
+            quad_resample<TW, TH, EDGE>(Q + L::P_GHR * QN, Q + L::P_GHB * QN, Q + L::P_DHR * QN, Q + L::P_DHB * QN,
+                                        Q + L::P_GVR * QN, Q + L::P_GVB * QN, i, j, qy0, qx0, H, W, v);
 #pragma unroll
-            for (int d = 0; d < 3; ++d) {
-                ri[d] = EDGE ? reflect101(fi + d - 1, hq) - qy0 : i + d - 1;
-                cj[d] = EDGE ? reflect101(fj + d - 1, wq) - qx0 : j + d - 1;
-            }
-            float gr[3][3], gb[3][3], dr[3][3], db[3][3];
-#pragma unroll
-            for (int a = 0; a < 3; ++a)
-#pragma unroll
-                for (int b = 0; b < 3; ++b) {
-                    int c = ri[a] * QW + cj[b];
-                    gr[a][b] = GR[c]; gb[a][b] = GB[c]; dr[a][b] = DR[c]; db[a][b] = DB[c];
-                }
-            float gw[4][4];
-            {
-                int wr[4], wc[4];
-                if (EDGE) {
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        wr[k] = (reflect101(2 * fi - 1 + k, H) >> 1) - qy0;
-                        wc[k] = (reflect101(2 * fj - 1 + k, W) >> 1) - qx0;
-                    }
-                } else {
-                    wr[0] = i - 1; wr[1] = i; wr[2] = i; wr[3] = i + 1;
-                    wc[0] = j - 1; wc[1] = j; wc[2] = j; wc[3] = j + 1;
-                }
-#pragma unroll
-                for (int a = 0; a < 4; ++a)
-#pragma unroll
-                    for (int b = 0; b < 4; ++b) {
-                        int c = wr[a] * QW + wc[b];
-                        const bool oddrow = (a & 1) == 0, oddcol = (b & 1) == 0;
-                        gw[a][b] = oddrow ? (oddcol ? GB[c] : G2[c]) : (oddcol ? G1[c] : GR[c]);
-                    }
-            }
-            float rp[4][2], ugr[4], udr[4], ugb[4], udb[4];
-#pragma unroll
-            for (int a = 0; a < 4; ++a) {
-                rp[a][0] = gauss_row(gw[a][0], gw[a][1], gw[a][2]);
-                rp[a][1] = gauss_row(gw[a][1], gw[a][2], gw[a][3]);
-            }
-            up_tl(gr, ugr); up_tl(dr, udr); up_br(gb, ugb); up_br(db, udb);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int a = k >> 1, b = k & 1;
-                float g = gw[a + 1][b + 1];
-                float hf = g - gauss_row(rp[a][b], rp[a + 1][b], rp[a + 2][b]);
-                Rgb v;
-                v.r = udr[k] + (ugr[k] + hf);
-                v.b = udb[k] + (ugb[k] + hf);
-                v.g = g;
-                stage_pixel<TW, TH>(out, p.st, p.g, p.c, 2 * oy + a, 2 * ox + b, v);
-            }
+            for (int k = 0; k < 4; ++k) stage_pixel<TW, TH>(out, p.st, p.g, p.c, 2 * oy + (k >> 1), 2 * ox + (k & 1), v[k]);
         }
     }
 }
