@@ -22,40 +22,63 @@ f32 = np.float32
 # ----------------------------------------------------------------------------------------------------------------
 # np.mean of a float32 colour plane (raw_correction.py:45)
 # ----------------------------------------------------------------------------------------------------------------
-def pairwise_leaf(a):
-    """NumPy's unrolled block sum of n <= 128 float32 values: eight strided partial sums, a fixed combine, then the tail."""
-    n = a.shape[0]
+def pairwise_leaves(a, offs, n):
+    """NumPy's unrolled block sum of n <= 128 float32 values, for the blocks a[o:o+n] of every o in `offs` at once: eight
+    strided partial sums, a fixed combine, then the tail."""
+    v = a[offs[:, None] + np.arange(n)]
     if n < 8:
-        res = f32(0.0)
+        res = np.zeros(len(offs), dtype=f32)
         for i in range(n):
-            res = f32(res + a[i])
+            res = (res + v[:, i]).astype(f32)
         return res
     m = n - (n % 8)
-    r = a[:m].reshape(-1, 8)
-    acc = r[0].copy()
-    for k in range(1, r.shape[0]):
-        acc = (acc + r[k]).astype(f32)
-    res = f32(f32(f32(acc[0] + acc[1]) + f32(acc[2] + acc[3])) + f32(f32(acc[4] + acc[5]) + f32(acc[6] + acc[7])))
+    r = v[:, :m].reshape(len(offs), -1, 8)
+    acc = r[:, 0].copy()
+    for k in range(1, r.shape[1]):
+        acc = (acc + r[:, k]).astype(f32)
+    res = (((acc[:, 0] + acc[:, 1]) + (acc[:, 2] + acc[:, 3])) + ((acc[:, 4] + acc[:, 5]) + (acc[:, 6] + acc[:, 7]))).astype(f32)
     for i in range(m, n):
-        res = f32(res + a[i])
+        res = (res + v[:, i]).astype(f32)
+    return res
+
+
+def _pairwise_level(a, groups):
+    """Sums of the runs of one recursion depth, {length: start offsets} -> {length: sums}.  The runs of the next depth are
+    grouped by length across parents, so every depth costs a few vector operations however many runs it has."""
+    nxt, plan, res = {}, [], {}
+    for n, offs in groups.items():
+        if n <= 128:
+            res[n] = pairwise_leaves(a, offs, n)
+            continue
+        n2 = n // 2
+        n2 -= n2 % 8
+        kids = []
+        for cn, co in ((n2, offs), (n - n2, offs + n2)):
+            parts = nxt.setdefault(cn, [])
+            kids.append((cn, sum(len(q) for q in parts)))
+            parts.append(co)
+        plan.append((n, len(offs), kids))
+    if nxt:
+        sub = _pairwise_level(a, {cn: np.concatenate(parts) for cn, parts in nxt.items()})
+        for n, k, ((ln, ls), (rn, rs)) in plan:
+            res[n] = (sub[ln][ls:ls + k] + sub[rn][rs:rs + k]).astype(f32)
     return res
 
 
 def pairwise_sum(a):
     """float32 sum in NumPy's order: recursive halving (left half rounded down to a multiple of 8) down to blocks of
-    at most 128 elements.  `a` is the plane in row-major order: bayer_to_rgbg's planes are strided views whose two
-    axes coalesce (bayer_chan_mixer.py:13-21), so np.mean sees one run of h*w elements."""
+    at most 128 elements, each half summed before the two are added.  `a` is the plane in row-major order: bayer_to_rgbg's
+    planes are strided views whose two axes coalesce (bayer_chan_mixer.py:13-21), so np.mean sees one run of h*w
+    elements."""
     a = np.ascontiguousarray(a, dtype=f32).ravel()
     n = a.shape[0]
-    if n <= 128:
-        return pairwise_leaf(a)
-    n2 = n // 2
-    n2 -= n2 % 8
-    return f32(pairwise_sum(a[:n2]) + pairwise_sum(a[n2:]))
+    return _pairwise_level(a, {n: np.zeros(1, dtype=np.int64)})[n][0]
 
 
 def plane_mean(p):
-    return f32(pairwise_sum(p) / f32(p.size))
+    """np.mean: the float32 sum divided by the integer count in float64, rounded to float32 once (numpy/_core/_methods.py,
+    _mean).  A float32 divisor gives the same bits only up to 2^24 elements, where float32(p.size) is still p.size."""
+    return f32(np.float64(pairwise_sum(p)) / p.size)
 
 
 # ----------------------------------------------------------------------------------------------------------------

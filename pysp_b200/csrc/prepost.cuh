@@ -6,7 +6,9 @@
 // most 128 elements are summed with eight strided accumulators, blocks are combined by recursive halving (left half
 // rounded down to a multiple of 8).  The tree only depends on the element count, so the host lays it out once
 // (PlaneSumPlan) and the device evaluates it in exactly that order: leaf_sum_kernel, then tree_sum_kernel level by
-// level.  The result is bit-identical to np.mean.
+// level.  np.mean then divides the float32 sum by the integer count in float64 and rounds the quotient to float32 once
+// (numpy/_core/_methods.py, _mean); tree_sum_kernel does the same.  (A float32 divisor agrees only up to 2^24 sites: above
+// that float32(n) may differ from n.)  The result is bit-identical to np.mean.
 #pragma once
 #include "pysp_common.cuh"
 
@@ -28,7 +30,6 @@ struct FlatParams {             // raw_correction.py:25-63
     float* out; long long out_pitch;
     int H, W;
     int clamp_high;
-    float n_f32;                // float32(h * w), the divisor of np.mean
     PlaneSumTables t;
     float* mean;                // [4] device
     int* stat;                  // [4][2]: ordered-int maximum of the finite quotients, number of quotients that are not +-inf
@@ -123,15 +124,16 @@ __global__ void __launch_bounds__(256) tree_level_kernel(PlaneSumTables t, int a
         val[t.n_leaves + k] = val[t.node_l[k]] + val[t.node_r[k]];
 }
 
-// one block = one plane: combine the remaining (narrow) levels in the order of NumPy's recursion, then mean = sum / float32(n)
-__global__ void __launch_bounds__(1024) tree_sum_kernel(PlaneSumTables t, int first_group, float n_f32, float* mean) {
+// one block = one plane: combine the remaining (narrow) levels in the order of NumPy's recursion, then
+// mean = float32(float64(sum) / float64(n)), the division np.mean does
+__global__ void __launch_bounds__(1024) tree_sum_kernel(PlaneSumTables t, int first_group, long long n, float* mean) {
     float* val = t.val + (long long)blockIdx.x * (t.n_leaves + t.n_nodes);
     for (int g = first_group; g < t.n_groups; ++g) {
         const int a = t.group_start[g], b = t.group_start[g + 1];
         for (int k = a + threadIdx.x; k < b; k += blockDim.x) val[t.n_leaves + k] = val[t.node_l[k]] + val[t.node_r[k]];
         __syncthreads();
     }
-    if (threadIdx.x == 0) mean[blockIdx.x] = val[t.n_leaves + t.n_nodes - 1] / n_f32;
+    if (threadIdx.x == 0) mean[blockIdx.x] = __double2float_rn(__ddiv_rn((double)val[t.n_leaves + t.n_nodes - 1], (double)n));
 }
 
 // work item of the two flat-field passes: four photosites of a row (two CFA sites, alternating)

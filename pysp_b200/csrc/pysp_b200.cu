@@ -705,7 +705,7 @@ int launch_plane_means(const float* mosaic, long long pitch, int H, int W, char*
         rc = check_launch("tree_level_kernel");
         if (rc) return rc;
     }
-    tree_sum_kernel<<<4, 1024, 0, stream>>>(t, g0, (float)n, (float*)(ws + lay.off_mean));
+    tree_sum_kernel<<<4, 1024, 0, stream>>>(t, g0, n, (float*)(ws + lay.off_mean));
     return check_launch("tree_sum_kernel");
 }
 }  // namespace
@@ -757,7 +757,7 @@ int pysp_flat_frame_correction(const float* sensor, int64_t sensor_pitch, const 
     cudaError_t e = cudaMemcpyAsync(ws + lay.off_stat, stat0, sizeof(stat0), cudaMemcpyHostToDevice, stream);
     if (e != cudaSuccess) return fail(PYSP_ERR_CUDA, "pysp_flat_frame_correction: %s", cudaGetErrorString(e));
     p.sensor = sensor; p.sensor_pitch = sensor_pitch; p.flat = flat; p.flat_pitch = flat_pitch; p.out = out; p.out_pitch = out_pitch;
-    p.H = H; p.W = W; p.clamp_high = clamp_high; p.n_f32 = (float)((long long)(H / 2) * (W / 2));
+    p.H = H; p.W = W; p.clamp_high = clamp_high;
     p.mean = (float*)(ws + lay.off_mean); p.stat = (int*)(ws + lay.off_stat);
     flat_stats_kernel<<<grid_for((long long)H * W, 256), 256, 0, stream>>>(p);
     rc = check_launch("flat_stats_kernel");

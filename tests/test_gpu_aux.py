@@ -27,10 +27,17 @@ def eng():
     return engine
 
 
-@pytest.mark.parametrize("shape", [(4, 6), (16, 16), (34, 50), (400, 600), (2000, 3000)])
+@pytest.mark.parametrize("shape", [(4, 6), (16, 16), (34, 50), (400, 600), (2000, 3000), (2, 2), (2, 258), (8194, 8194),
+                                   (8662, 11550)])
 def test_plane_means_are_numpys(eng, shape):
-    rng = np.random.default_rng(shape[0])
-    m = (rng.random(shape) * rng.choice([1e-3, 1.0, 50.0], size=shape)).astype(np.float32)
+    """(2, 258): 129 sites, one 128-element leaf and a tail.  8194 x 8194 (4097^2 = 2^24 + 8193 sites) and 8662 x 11550
+    (25 011 525): planes above 2^24 sites, where np.mean's float64 division by the count differs from a division by
+    float32(n); their wide tree levels run in tree_level_kernel."""
+    if shape[0] * shape[1] > 2 ** 26:
+        m = np.random.default_rng(0).random(shape, dtype=np.float32)
+    else:
+        rng = np.random.default_rng(shape[0])
+        m = (rng.random(shape) * rng.choice([1e-3, 1.0, 50.0], size=shape)).astype(np.float32)
     got = eng.bayer_plane_means(eng.to_device(m)).cpu().numpy()
     evens, odds = m[0::2, :].astype(np.float32), m[1::2, :].astype(np.float32)      # bayer_chan_mixer.py:13-21
     want = np.array([np.mean(evens[:, 0::2]), np.mean(evens[:, 1::2]), np.mean(odds[:, 1::2]), np.mean(odds[:, 0::2])], np.float32)

@@ -118,7 +118,8 @@ def test_identity_and_errors(eng):
     # strong magnification / shear: the source windows of a block no longer fit the shared-memory patch and the kernel
     # gathers from global memory instead -- same bits as the two-step form (table in HBM, then remap) either way
     big = torch.rand((200, 328, 3), device="cuda")
-    for k in ((2.2, -0.3, 0.1, 0.0, 0.05, -0.04), (0.45, 0.2, 0.0, 0.0, 0.0, 0.0), (1.01, -0.02, 0.0, 0.0, 0.3, 0.25)):
+    for k in ((2.2, -0.3, 0.1, 0.0, 0.05, -0.04), (0.45, 0.2, 0.0, 0.0, 0.0, 0.0), (1.01, -0.02, 0.0, 0.0, 0.3, 0.25),
+              (1.3, 0.5, 0.0, 0.0, 0.0, 0.0)):
         fused = eng.warp_rectilinear(big, [k] * 3, (0.47, 0.52), 1.0)
         for i in range(3):
             two = eng.remap_lanczos4(big, i, eng.warp_table(200, 328, k, (0.47, 0.52), 1.0))
