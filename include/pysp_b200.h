@@ -236,6 +236,42 @@ int pysp_warp_rectilinear_apply(const float* src, float* dst, int32_t height, in
                                 float cam_center_norm_x, float cam_center_norm_y, float scale, const float* prior,
                                 const float* lanczos_tab, void* stream);
 
+/* ---- baseline JPEG of the PYSP_OUT_YCC420_U8 planes --------------------------------------------------------------------
+ *
+ * pysp_jpeg_encode_ycc420 writes one complete JFIF file byte-identical to libjpeg(-turbo)'s encode of the same planes with
+ * its defaults, i.e. Pillow's
+ *     Image.merge("YCbCr", [Y, upsample2x2(Cb), upsample2x2(Cr)]).save(f, "JPEG", quality=quality, subsampling=2)
+ * When W is a multiple of 16 and the planes are PYSP_OUT_YCC420_U8 of a develop, that is also byte-identical to the JPEG
+ * libjpeg writes from the PYSP_OUT_SRGB_U8 image of the same call (for other widths libjpeg pads the chroma's right edge from
+ * full-resolution chroma, which the planes do not hold).  What it does, all in integers (tests/jpeg_ref.py restates it):
+ *  - markers SOI, APP0 (JFIF 1.01, density 1:1, no units), DQT luma, DQT chroma (8-bit, zigzag order), SOF0, DHT DC0, AC0,
+ *    DC1, AC1 (the standard tables of Annex K.3), SOS, the entropy-coded data, EOI; MCU = Y00 Y01 Y10 Y11 Cb Cr, no restarts;
+ *  - quantisation tables: scale = quality < 50 ? 5000/quality : 200 - 2*quality, clamp((std*scale + 50)/100, 1, 255) on
+ *    the Annex K.1 tables;
+ *  - jfdctint.c ISLOW forward DCT of x - 128; coefficient c is quantised as sign(c) * ((|c| + d/2) / d), d = 8*qtab[k];
+ *  - each plane is padded to whole 8x8 blocks by repeating its last column and row; a Y slot of an MCU outside the Y blocks
+ *    is a dummy block: AC zero, DC = the DC of the block before it in the MCU;
+ *  - DC prediction per component across the scan, ZRL for runs of 16 zeros, EOB for trailing zeros, the last byte padded
+ *    with 1-bits, 0x00 after every 0xFF of the entropy-coded data.
+ * y: [height][width] (pitch y_pitch >= width), cb / cr: [height/2][width/2] (one pitch chroma_pitch >= width/2); height and
+ * width even, 2..65535; quality 1..100.  out: >= pysp_jpeg_max_bytes(height, width) bytes (out_capacity); *out_len (a DEVICE
+ * int64) receives the file's length, and no byte of `out` past it is written.  workspace: >= pysp_jpeg_workspace_bytes.
+ * Every argument is checked before any CUDA call (PYSP_ERR_INVALID).  The header and the quantisation tables are written by a
+ * kernel and the Huffman tables live in constant memory: a call makes no host <-> device copy and can be captured in a CUDA
+ * graph. */
+/* The worst case of the file.  A block codes its DC difference (category <= 11: a code of at most 11 bits plus 11 magnitude
+ * bits) and its 63 AC coefficients; each AC symbol (a code of at most 16 bits plus at most 10 magnitude bits) accounts for at
+ * least one coefficient, and so do ZRL (16 coefficients) and EOB (at least one), so a block takes at most
+ * 11 + 11 + 63 * (16 + 10) = 1660 bits.  With 6 blocks per MCU the entropy-coded data is at most ceil(6 * MCUs * 1660 / 8)
+ * bytes (the padding completes the last byte); stuffing at most doubles it.  Plus the 623-byte header and the 2-byte EOI.
+ * 0 for an invalid size. */
+int64_t pysp_jpeg_max_bytes(int32_t height, int32_t width);
+/* Bytes of device workspace pysp_jpeg_encode_ycc420 needs (0 for an invalid size). */
+int64_t pysp_jpeg_workspace_bytes(int32_t height, int32_t width);
+int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t chroma_pitch,
+                            int32_t height, int32_t width, int32_t quality, uint8_t* out, int64_t out_capacity,
+                            int64_t* out_len, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* Bench instrumentation (no reference counterpart): when enabled, pysp_develop brackets each kernel launch
  * with CUDA events on the launching stream; collect() synchronises them and returns, per kernel slot
  * (0 = ahd_select_kernel, 1 = median_stage_kernel; 4 slots), the summed device milliseconds and launch

@@ -102,6 +102,13 @@ def lib():
     L.pysp_warp_rectilinear_apply.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float),
                                               C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pysp_warp_rectilinear_apply.restype = C.c_int
+    L.pysp_jpeg_max_bytes.argtypes = [C.c_int32, C.c_int32]
+    L.pysp_jpeg_max_bytes.restype = C.c_int64
+    L.pysp_jpeg_workspace_bytes.argtypes = [C.c_int32, C.c_int32]
+    L.pysp_jpeg_workspace_bytes.restype = C.c_int64
+    L.pysp_jpeg_encode_ycc420.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
+                                          C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    L.pysp_jpeg_encode_ycc420.restype = C.c_int
     L.pysp_timing_enable.argtypes = [C.c_int32]
     L.pysp_timing_enable.restype = None
     L.pysp_timing_collect.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int64)]

@@ -21,6 +21,7 @@
 #include "pointwise.cuh"
 #include "prepost.cuh"
 #include "warp.cuh"
+#include "jpeg.cuh"
 #include "develop_plan.h"
 
 namespace pysp {
@@ -881,6 +882,57 @@ int pysp_warp_rectilinear_apply(const float* src, float* dst, int32_t H, int32_t
     const long long cap = 148LL * 32;
     warp_apply_kernel<<<(int)(tiles < cap ? tiles : cap), 256, 0, (cudaStream_t)stream>>>(p);
     return check_launch("warp_apply_kernel");
+}
+
+}  // extern "C"
+
+// ---- baseline JPEG of YCbCr 4:2:0 planes (jpeg.cuh) ------------------------------------------------------------------
+extern "C" {
+
+int64_t pysp_jpeg_max_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_max_bytes(H, W) : 0; }
+
+int64_t pysp_jpeg_workspace_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_layout(H, W, nullptr, nullptr) : 0; }
+
+int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t chroma_pitch, int32_t H,
+                            int32_t W, int32_t quality, uint8_t* out, int64_t out_capacity, int64_t* out_len, void* workspace,
+                            int64_t workspace_bytes, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    JpegParams p;
+    if (plan_jpeg(y, y_pitch, cb, cr, chroma_pitch, H, W, quality, out, out_capacity, out_len, workspace, workspace_bytes, &p, g_err,
+                  sizeof(g_err)))
+        return PYSP_ERR_INVALID;
+    int rc = ensure_device();
+    if (rc) return rc;
+    const long long cap = 148LL * 8;                     // fixed grids of the kernels whose item count is on the device
+    const int block_grid = (int)((p.n_blocks + JPEG_THREADS - 1) / JPEG_THREADS);
+    const long long bchunks = (p.n_blocks + JPEG_SCAN_CHUNK - 1) / JPEG_SCAN_CHUNK;
+    const long long fchunks = (p.max_items + JPEG_SCAN_CHUNK - 1) / JPEG_SCAN_CHUNK;
+    const JpegScan bscan = {p.bits, p.boff, p.bchunk, p.totals, p.n_blocks, nullptr};
+    const JpegScan fscan = {p.ffcnt, p.foff, p.fchunk, p.totals + 1, 0, p.totals};
+    jpeg_header_kernel<<<1, JPEG_THREADS, 0, stream>>>(p);
+    if ((rc = check_launch("jpeg_header_kernel"))) return rc;
+    jpeg_block_kernel<<<block_grid, JPEG_THREADS, 0, stream>>>(p);
+    if ((rc = check_launch("jpeg_block_kernel"))) return rc;
+    jpeg_scan_reduce_kernel<<<(int)std::min(bchunks, cap), JPEG_THREADS, 0, stream>>>(bscan);
+    if ((rc = check_launch("jpeg_scan_reduce_kernel"))) return rc;
+    jpeg_scan_top_kernel<<<1, JPEG_THREADS, 0, stream>>>(bscan);
+    if ((rc = check_launch("jpeg_scan_top_kernel"))) return rc;
+    jpeg_scan_down_kernel<<<(int)std::min(bchunks, cap), JPEG_THREADS, 0, stream>>>(bscan);
+    if ((rc = check_launch("jpeg_scan_down_kernel"))) return rc;
+    jpeg_zero_kernel<<<(int)cap, JPEG_THREADS, 0, stream>>>(p);
+    if ((rc = check_launch("jpeg_zero_kernel"))) return rc;
+    jpeg_pack_kernel<<<block_grid, JPEG_THREADS, 0, stream>>>(p);
+    if ((rc = check_launch("jpeg_pack_kernel"))) return rc;
+    jpeg_count_kernel<<<(int)cap, JPEG_THREADS, 0, stream>>>(p);
+    if ((rc = check_launch("jpeg_count_kernel"))) return rc;
+    jpeg_scan_reduce_kernel<<<(int)std::min(fchunks, cap), JPEG_THREADS, 0, stream>>>(fscan);
+    if ((rc = check_launch("jpeg_scan_reduce_kernel"))) return rc;
+    jpeg_scan_top_kernel<<<1, JPEG_THREADS, 0, stream>>>(fscan);
+    if ((rc = check_launch("jpeg_scan_top_kernel"))) return rc;
+    jpeg_scan_down_kernel<<<(int)std::min(fchunks, cap), JPEG_THREADS, 0, stream>>>(fscan);
+    if ((rc = check_launch("jpeg_scan_down_kernel"))) return rc;
+    jpeg_emit_kernel<<<(int)cap, JPEG_THREADS, 0, stream>>>(p);
+    return check_launch("jpeg_emit_kernel");
 }
 
 }  // extern "C"

@@ -231,6 +231,56 @@ def develop(mosaic, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white
     return out_tensor
 
 
+def jpeg_max_bytes(height, width):
+    """pysp_jpeg_max_bytes: the largest file encode_jpeg can write for an even-sized frame"""
+    n = int(_capi.lib().pysp_jpeg_max_bytes(int(height), int(width)))
+    if n <= 0:
+        raise ValueError("jpeg_max_bytes: height and width must be even, 2..65535 (got %dx%d)" % (height, width))
+    return n
+
+
+def encode_jpeg(planes, quality=75, out_tensor=None, stream=None):
+    """Baseline JPEG of YCbCr 4:2:0 planes on the device (include/pysp_b200.h, pysp_jpeg_encode_ycc420): byte-identical to
+    libjpeg's encode of the planes (Pillow: Image.merge("YCbCr", [Y, Cb, Cr upsampled 2x2]).save(f, "JPEG", quality=quality,
+    subsampling=2)); when W is a multiple of 16, to libjpeg's JPEG of the srgb_u8 image the planes were developed from.
+
+    planes      (y, cb, cr): uint8 CUDA views [H, W], [H/2, W/2], [H/2, W/2] with unit column stride, any row pitches (Cb and
+                Cr sharing one), e.g. what develop(out="ycc420") returns.
+    out_tensor  optional flat uint8 CUDA tensor of >= jpeg_max_bytes(H, W) bytes.
+    Returns (buf, n): `buf` the uint8 CUDA tensor holding the file in its first n bytes, `n` a 0-d int64 CUDA tensor.  Nothing
+    is synchronised: read n (e.g. n.item()) after the stream has reached it.
+    """
+    require_cuda()
+    L = _capi.lib()
+    ok = isinstance(planes, (tuple, list)) and len(planes) == 3
+    if ok:
+        y, cb, cr = planes
+        ok = all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.uint8 and t.dim() == 2 and t.stride(1) == 1
+                 for t in planes)
+    if ok:
+        H, W = y.shape
+        ok = H % 2 == 0 and W % 2 == 0 and cb.shape == cr.shape == (H // 2, W // 2) and cb.stride(0) == cr.stride(0) and \
+            cb.device == y.device and cr.device == y.device
+    if not ok:
+        raise ValueError("encode_jpeg: planes must be (y, cb, cr) uint8 CUDA views [H, W], [H/2, W/2], [H/2, W/2] of even H, W "
+                         "on one device, with unit column stride and one chroma pitch")
+    dev = y.device
+    cap = jpeg_max_bytes(H, W)
+    with _on(dev, stream):
+        if out_tensor is None:
+            out_tensor = torch.empty(cap, dtype=torch.uint8, device=dev)
+        elif (not out_tensor.is_cuda or out_tensor.dtype != torch.uint8 or out_tensor.dim() != 1 or not out_tensor.is_contiguous()
+              or out_tensor.device != dev):
+            raise ValueError("encode_jpeg: out_tensor must be a flat contiguous uint8 CUDA tensor on the planes' device")
+        nws = int(L.pysp_jpeg_workspace_bytes(H, W))
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        n = torch.empty((), dtype=torch.int64, device=dev)
+        _capi.check(L.pysp_jpeg_encode_ycc420(y.data_ptr(), y.stride(0), cb.data_ptr(), cr.data_ptr(), cb.stride(0), H, W,
+                                              int(quality), out_tensor.data_ptr(), out_tensor.numel(), n.data_ptr(),
+                                              ws.data_ptr(), nws, _stream_ptr(stream)))
+    return out_tensor, n
+
+
 def normalize(raw, black, white, stream=None):
     """bayer_normalize on the device: uint16 [H,W] -> float32 [H,W]."""
     require_cuda()

@@ -8,6 +8,11 @@ with the SMs).  No CPU computation is involved.
 
 With out="ycc420" each output is one flat I420 buffer of H*W*3/2 bytes (Y, then Cb, then Cr; engine.i420_planes gives the
 three planes of it), so one copy moves a frame.
+
+With out="jpeg" each frame is developed into device ycc420 planes and encoded on the device (engine.encode_jpeg, quality
+`jpeg_quality`); its length goes to pinned host memory, and once that has landed exactly that many bytes are copied into the
+frame's output.  The host waits for frame i's length only after frame i + depth - 1 has been queued, so the later frames' work
+keeps the GPU busy while it waits.  `run` returns the lengths.
 """
 import torch
 
@@ -16,26 +21,36 @@ from . import engine
 
 class FramePipeline:
     def __init__(self, height, width, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white=None,
-                 hdr=False, gamma=False, out="lin", device=None, depth=3):
+                 hdr=False, gamma=False, out="lin", device=None, depth=3, jpeg_quality=75):
         engine.require_cuda()
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         self.h, self.w = int(height), int(width)
+        self.jpeg = out == "jpeg"
+        self.jpeg_quality = int(jpeg_quality)
+        planes = out in ("ycc420", "jpeg")
         self.kw = dict(wb=wb, cam_to_srgb=cam_to_srgb, stages=stages, pattern=pattern, black=black, white=white,
-                       hdr=hdr, gamma=gamma, out=out)
-        self.out_dtype = engine._OUT_DTYPES[engine._OUT_KINDS[out]]
-        self.out_shape = (engine.i420_bytes(self.h, self.w),) if out == "ycc420" else (self.h, self.w, 3)
+                       hdr=hdr, gamma=gamma, out="ycc420" if self.jpeg else out)
+        self.out_dtype = engine._OUT_DTYPES[engine._OUT_KINDS[self.kw["out"]]]
+        self.out_shape = (engine.i420_bytes(self.h, self.w),) if planes else (self.h, self.w, 3)
         self.depth = depth
         with torch.cuda.device(self.device):
             self.streams = [torch.cuda.Stream() for _ in range(depth)]
             self.d_in = [torch.empty((self.h, self.w), dtype=torch.int16, device=self.device) for _ in range(depth)]
             self.d_out = [torch.empty(self.out_shape, dtype=self.out_dtype, device=self.device) for _ in range(depth)]
         # what develop writes into: the output tensor itself, or the three planes over the flat I420 buffer
-        self.d_dst = [engine.i420_planes(d, self.h, self.w) if out == "ycc420" else d for d in self.d_out]
+        self.d_dst = [engine.i420_planes(d, self.h, self.w) if planes else d for d in self.d_out]
+        if self.jpeg:
+            self.jpeg_bytes = engine.jpeg_max_bytes(self.h, self.w)
+            with torch.cuda.device(self.device):
+                self.d_jpeg = [torch.empty(self.jpeg_bytes, dtype=torch.uint8, device=self.device) for _ in range(depth)]
 
     def pinned_input(self):
         return torch.empty((self.h, self.w), dtype=torch.int16).pin_memory()
 
     def pinned_output(self):
+        """a host buffer for one output; for out="jpeg" sized to the largest file (engine.jpeg_max_bytes)"""
+        if self.jpeg:
+            return torch.empty(self.jpeg_bytes, dtype=torch.uint8).pin_memory()
         return torch.empty(self.out_shape, dtype=self.out_dtype).pin_memory()
 
     def h2d_bytes(self):
@@ -46,8 +61,10 @@ class FramePipeline:
 
     def run(self, host_frames, host_outputs):
         """host_frames[i] (int16/uint16 bits, ideally pinned) -> host_outputs[i] (pinned).  Returns after
-        every output has landed in host memory."""
+        every output has landed in host memory; for out="jpeg" the list of file lengths (host_outputs[i][:n[i]])."""
         assert len(host_frames) == len(host_outputs)
+        if self.jpeg:
+            return self._run_jpeg(host_frames, host_outputs)
         with torch.cuda.device(self.device):
             for i, (src, dst) in enumerate(zip(host_frames, host_outputs)):
                 k = i % self.depth
@@ -59,16 +76,51 @@ class FramePipeline:
             for s in self.streams:
                 s.synchronize()
 
-    def run_copies_only(self, host_frames, host_outputs):
+    def _run_jpeg(self, host_frames, host_outputs):
+        lens = [torch.empty((), dtype=torch.int64).pin_memory() for _ in host_frames]
+        landed = [None] * len(host_frames)
+        out = [0] * len(host_frames)
+
+        def download(i):                   # frame i's length has been copied: copy exactly that many bytes
+            landed[i].synchronize()
+            n = out[i] = int(lens[i])
+            k = i % self.depth
+            with torch.cuda.stream(self.streams[k]):
+                host_outputs[i][:n].copy_(self.d_jpeg[k][:n], non_blocking=True)
+
+        with torch.cuda.device(self.device):
+            for i, src in enumerate(host_frames):
+                k = i % self.depth
+                s = self.streams[k]
+                with torch.cuda.stream(s):
+                    self.d_in[k].copy_(src, non_blocking=True)
+                    engine.develop(self.d_in[k], out_tensor=self.d_dst[k], stream=s, **self.kw)
+                    _, n = engine.encode_jpeg(self.d_dst[k], self.jpeg_quality, out_tensor=self.d_jpeg[k], stream=s)
+                    lens[i].copy_(n, non_blocking=True)
+                    landed[i] = torch.cuda.Event()
+                    landed[i].record(s)
+                if i - (self.depth - 1) >= 0:
+                    download(i - (self.depth - 1))
+            for i in range(max(0, len(host_frames) - (self.depth - 1)), len(host_frames)):
+                download(i)
+            for s in self.streams:
+                s.synchronize()
+        return out
+
+    def run_copies_only(self, host_frames, host_outputs, nbytes=None):
         """The copies of `run` without the kernels: the same pinned buffers, byte counts, streams and order, one
         cudaMemcpyAsync per copy (what `Tensor.copy_(non_blocking=True)` issues between pinned host and device memory).
-        Its rate is the ceiling the host <-> device path of this box puts on `run`."""
+        Its rate is the ceiling the host <-> device path of this box puts on `run`.  For out="jpeg", `nbytes[i]` is the
+        length of frame i's file (what `run` returned): that many bytes are copied down."""
         assert len(host_frames) == len(host_outputs)
         with torch.cuda.device(self.device):
             for i, (src, dst) in enumerate(zip(host_frames, host_outputs)):
                 k = i % self.depth
                 with torch.cuda.stream(self.streams[k]):
                     self.d_in[k].copy_(src, non_blocking=True)
-                    dst.copy_(self.d_out[k], non_blocking=True)
+                    if self.jpeg:
+                        dst[:nbytes[i]].copy_(self.d_jpeg[k][:nbytes[i]], non_blocking=True)
+                    else:
+                        dst.copy_(self.d_out[k], non_blocking=True)
             for s in self.streams:
                 s.synchronize()
