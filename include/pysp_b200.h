@@ -17,9 +17,6 @@
  *        CUDA graph);
  *      . the verdict of the last normalisation-division check (exhaustive over the 65536 sensor codes of one
  *        level set; re-done when the levels change);
- *      . for pysp_bayer_plane_means / pysp_flat_frame_correction, the NumPy summation trees of the last 8
- *        plane sizes (host memory, oldest dropped); their tables are copied into the caller's workspace with
- *        cudaMemcpyAsync from pageable host memory on every call (so these two are not graph-capturable);
  *      . the event pairs of the bench instrumentation while pysp_timing_enable(1) is in effect;
  *      . the test hook PYSP_DISABLE_TMA, read once per process;
  *  - return value: PYSP_OK or a negative code; pysp_last_error() returns the calling thread's message.

@@ -4,25 +4,54 @@
 // flat_frame_correction (raw_correction.py:25-63) needs np.mean of each CFA plane of the flat field in float32, and
 // NumPy's float32 sum is a *pairwise* sum with a fixed shape (loops_utils.h.src, @TYPE@_pairwise_sum): blocks of at
 // most 128 elements are summed with eight strided accumulators, blocks are combined by recursive halving (left half
-// rounded down to a multiple of 8).  The tree only depends on the element count, so the host lays it out once
-// (PlaneSumPlan) and the device evaluates it in exactly that order: leaf_sum_kernel, then tree_sum_kernel level by
-// level.  np.mean then divides the float32 sum by the integer count in float64 and rounds the quotient to float32 once
-// (numpy/_core/_methods.py, _mean); tree_sum_kernel does the same.  (A float32 divisor agrees only up to 2^24 sites: above
-// that float32(n) may differ from n.)  The result is bit-identical to np.mean.
+// rounded down to a multiple of 8).  The tree only depends on the element count, and a node's elements follow from its
+// position: node (d, i), the i-th node from the left at depth d, is reached from the root by applying NumPy's split once
+// per bit of i (sum_node).  So the device evaluates the tree in exactly NumPy's order without a table: leaf_sum_kernel,
+// then tree_level_kernel / tree_sum_kernel level by level.  np.mean then divides the float32 sum by the integer count in
+// float64 and rounds the quotient to float32 once (numpy/_core/_methods.py, _mean); tree_sum_kernel does the same.  (A
+// float32 divisor agrees only up to 2^24 sites: above that float32(n) may differ from n.)  The result is bit-identical
+// to np.mean.
 #pragma once
 #include "pysp_common.cuh"
 
 namespace pysp {
 
-struct PlaneSumTables {         // device pointers into the caller's workspace
-    const int* leaf_off;        // [n_leaves] first plane element of the leaf
-    const int* leaf_len;        // [n_leaves] 1..128
-    const int* node_l;          // [n_nodes] value index of the left child (leaves are 0..n_leaves-1, nodes follow)
-    const int* node_r;
-    const int* group_start;     // [n_groups + 1] nodes of one group are independent (same height)
-    int n_leaves, n_nodes, n_groups;
-    float* val;                 // [4][n_leaves + n_nodes]
+// NumPy's pairwise-sum tree of one plane of n elements.  With n = 8K + t, every left part is a whole number of 8-element
+// units (floor(k/2) of a node's k), so the sizes of the nodes at one depth differ by at most one unit plus the t-element
+// tail, which stays on the right spine, the largest node of every depth.  Every leaf therefore sits on depth D, where the
+// right spine first holds at most 128 elements, or on D - 1, and every node on level L = max(D - 1, 0) is a leaf or the
+// parent of two leaves.  leaf_sum_kernel writes level L, the levels above it are sums of two children.  Values are kept
+// in heap order: node (d, i) in slot s = 2^d - 1 + i, its children in slots 2s + 1 and 2s + 2, 2^(L+1) - 1 slots per plane.
+struct PlaneSumTree {
+    long long n;
+    int L;
+    float* val;                 // [4][2^(L+1) - 1] in the caller's workspace
 };
+
+// NumPy's split of a run of more than 128 elements: the left part is half of it, rounded down to a multiple of 8
+template <typename T> PYSP_HOSTDEV inline T pairwise_left(T n) { return n / 2 - (n / 2) % 8; }
+
+PYSP_HOSTDEV inline PlaneSumTree plane_sum_tree(long long n, float* val) {
+    int D = 0;
+    for (long long r = n; r > 128; r -= pairwise_left(r)) ++D;          // down the right spine
+    return {n, D > 0 ? D - 1 : 0, val};
+}
+
+struct SumNode { int first, count; };   // plane elements [first, first + count); a leaf iff count <= 128
+
+// node (d, i): NumPy's split applied along the path from the root, bit b of i choosing the right part at depth d - b
+PYSP_HD SumNode sum_node(const PlaneSumTree& s, int d, int i) {
+    SumNode e = {0, (int)s.n};
+    for (int b = d - 1; b >= 0; --b) {
+        const int l = pairwise_left(e.count);
+        if ((i >> b) & 1) { e.first += l; e.count -= l; } else e.count = l;
+    }
+    return e;
+}
+
+// node e on level L is summed as two runs [first, first + l) and [first + l, first + count): a leaf as itself and an empty
+// run, an internal node as its two leaf children
+PYSP_HD int leaf_part(const SumNode& e) { return e.count > 128 ? pairwise_left(e.count) : e.count; }
 
 struct FlatParams {             // raw_correction.py:25-63
     const float* sensor; long long sensor_pitch;
@@ -30,7 +59,6 @@ struct FlatParams {             // raw_correction.py:25-63
     float* out; long long out_pitch;
     int H, W;
     int clamp_high;
-    PlaneSumTables t;
     float* mean;                // [4] device
     int* stat;                  // [4][2]: ordered-int maximum of the finite quotients, number of quotients that are not +-inf
 };
@@ -74,66 +102,76 @@ __device__ __forceinline__ float plane_elem(const float* base, long long pitch, 
     return *((const float*)((const char*)base + (long long)(2 * i + py) * pitch) + 2 * j + px);
 }
 
-// eight lanes = one leaf of one plane, evaluated exactly as NumPy's unrolled block sum: lane j owns the strided partial
-// sum r[j]; the fixed combine ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) is an xor-butterfly (float addition commutes), the
-// tail elements are added by lane 0 in order.  Eight consecutive plane elements are 64 contiguous bytes of the mosaic.
-__global__ void __launch_bounds__(256) leaf_sum_kernel(const float* mosaic, long long pitch, int W, PlaneSumTables t) {
+// eight lanes sum the leaf [off, off + n) of one plane (n <= 128, 0 for nothing) exactly as NumPy's unrolled block sum:
+// lane j owns the strided partial sum r[j]; the fixed combine ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) is an xor-butterfly
+// (float addition commutes), the tail elements are added by lane 0 in order.  Eight consecutive plane elements are 64
+// contiguous bytes of the mosaic.  Every lane of the warp calls it; the sum is lane 0's result.
+__device__ __forceinline__ float leaf_sum(const float* mosaic, long long pitch, int w, int py, int px, int off, int n, int lane8) {
+    float res = 0.0f;
+    if (n < 8) {
+        if (lane8 == 0) for (int i = 0; i < n; ++i) res = res + plane_elem(mosaic, pitch, w, py, px, off + i);
+    } else {
+        // walk (row, column) of the plane incrementally: one division per leaf instead of one per element
+        int e = off + lane8, i = e / w, j = e - i * w;
+        float r = *((const float*)((const char*)mosaic + (long long)(2 * i + py) * pitch) + 2 * j + px);
+        for (int k = 8; k < n - (n % 8); k += 8) {
+            j += 8;
+            while (j >= w) { j -= w; ++i; }
+            r = r + *((const float*)((const char*)mosaic + (long long)(2 * i + py) * pitch) + 2 * j + px);
+        }
+        res = r;
+    }
+    // groups with n < 8 carry zeros that only lane 0's own sum replaces
+    float s = res;
+    s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 1);
+    s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 2);
+    s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 4);
+    if (lane8 == 0 && n >= 8) {
+        res = s;
+        for (int i = n - (n % 8); i < n; ++i) res = res + plane_elem(mosaic, pitch, w, py, px, off + i);
+    }
+    return res;
+}
+
+// one work item = eight lanes = node (L, i) of one plane: a leaf, or two leaves summed one after the other and added
+// left + right, as NumPy's recursion adds them
+__global__ void __launch_bounds__(256) leaf_sum_kernel(const float* mosaic, long long pitch, int W, PlaneSumTree t) {
     const int w = W >> 1;
-    const int total = 4 * t.n_leaves;
+    const int total = 4 << t.L;                                 // a multiple of 4: whole warps stay together for the shuffles
     const int lane8 = threadIdx.x & 7;
     const int groups = (gridDim.x * blockDim.x) >> 3;
-    const int total_pad = (total + 3) / 4 * 4;                 // whole warps stay together for the shuffles
-    for (int id = (blockIdx.x * blockDim.x + threadIdx.x) >> 3; id < total_pad; id += groups) {
-        const bool live = id < total;
-        const int p = live ? id / t.n_leaves : 0, leaf = live ? id - p * t.n_leaves : 0;
+    for (int id = (blockIdx.x * blockDim.x + threadIdx.x) >> 3; id < total; id += groups) {
+        const int p = id >> t.L, i = id & ((1 << t.L) - 1);
         const int py = plane_py(p), px = plane_px(p);
-        const int off = t.leaf_off[leaf], n = live ? t.leaf_len[leaf] : 0;
-        float res = 0.0f;
-        if (n < 8) {
-            if (lane8 == 0) for (int i = 0; i < n; ++i) res = res + plane_elem(mosaic, pitch, w, py, px, off + i);
-        } else {
-            // walk (row, column) of the plane incrementally: one division per leaf instead of one per element
-            int e = off + lane8, i = e / w, j = e - i * w;
-            float r = *((const float*)((const char*)mosaic + (long long)(2 * i + py) * pitch) + 2 * j + px);
-            for (int k = 8; k < n - (n % 8); k += 8) {
-                j += 8;
-                while (j >= w) { j -= w; ++i; }
-                r = r + *((const float*)((const char*)mosaic + (long long)(2 * i + py) * pitch) + 2 * j + px);
-            }
-            res = r;
-        }
-        // every lane of the warp takes part; groups with n < 8 carry zeros that only lane 0's own sum replaces
-        float s = res;
-        s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 1);
-        s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 2);
-        s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 4);
-        if (lane8 == 0 && live) {
-            if (n >= 8) {
-                res = s;
-                for (int i = n - (n % 8); i < n; ++i) res = res + plane_elem(mosaic, pitch, w, py, px, off + i);
-            }
-            t.val[(long long)p * (t.n_leaves + t.n_nodes) + leaf] = res;
-        }
+        const SumNode e = sum_node(t, t.L, i);
+        const int l = leaf_part(e);
+        const float a = leaf_sum(mosaic, pitch, w, py, px, e.first, l, lane8);
+        const float b = leaf_sum(mosaic, pitch, w, py, px, e.first + l, e.count - l, lane8);
+        if (lane8 == 0) t.val[(long long)p * ((2 << t.L) - 1) + (1 << t.L) - 1 + i] = l < e.count ? a + b : a;
     }
 }
 
-// one wide level of the recursion tree (nodes [a, b) are independent), all four planes: blockIdx.y = plane
-__global__ void __launch_bounds__(256) tree_level_kernel(PlaneSumTables t, int a, int b) {
-    float* val = t.val + (long long)blockIdx.y * (t.n_leaves + t.n_nodes);
-    for (int k = a + blockIdx.x * blockDim.x + threadIdx.x; k < b; k += gridDim.x * blockDim.x)
-        val[t.n_leaves + k] = val[t.node_l[k]] + val[t.node_r[k]];
+// one wide level d of the tree (its 2^d nodes are independent), all four planes: blockIdx.y = plane.  Node = left child
+// + right child, as NumPy's recursion adds them.
+__global__ void __launch_bounds__(256) tree_level_kernel(PlaneSumTree t, int d) {
+    float* val = t.val + (long long)blockIdx.y * ((2 << t.L) - 1);
+    for (int s = (1 << d) - 1 + blockIdx.x * blockDim.x + threadIdx.x; s < (2 << d) - 1; s += gridDim.x * blockDim.x)
+        val[s] = val[2 * s + 1] + val[2 * s + 2];
 }
 
-// one block = one plane: combine the remaining (narrow) levels in the order of NumPy's recursion, then
-// mean = float32(float64(sum) / float64(n)), the division np.mean does
-__global__ void __launch_bounds__(1024) tree_sum_kernel(PlaneSumTables t, int first_group, long long n, float* mean) {
-    float* val = t.val + (long long)blockIdx.x * (t.n_leaves + t.n_nodes);
-    for (int g = first_group; g < t.n_groups; ++g) {
-        const int a = t.group_start[g], b = t.group_start[g + 1];
-        for (int k = a + threadIdx.x; k < b; k += blockDim.x) val[t.n_leaves + k] = val[t.node_l[k]] + val[t.node_r[k]];
+// one block = one plane: combine levels d0 .. 0 (the narrow top of the tree), then mean = float32(float64(sum) /
+// float64(n)), the division np.mean does.  With `stat` (flat-field correction) it also resets the plane's statistics words
+// that flat_stats_kernel, launched next on the same stream, accumulates into.
+__global__ void __launch_bounds__(1024) tree_sum_kernel(PlaneSumTree t, int d0, float* mean, int* stat) {
+    float* val = t.val + (long long)blockIdx.x * ((2 << t.L) - 1);
+    for (int d = d0; d >= 0; --d) {
+        for (int s = (1 << d) - 1 + threadIdx.x; s < (2 << d) - 1; s += blockDim.x) val[s] = val[2 * s + 1] + val[2 * s + 2];
         __syncthreads();
     }
-    if (threadIdx.x == 0) mean[blockIdx.x] = __double2float_rn(__ddiv_rn((double)val[t.n_leaves + t.n_nodes - 1], (double)n));
+    if (threadIdx.x == 0) {
+        mean[blockIdx.x] = __double2float_rn(__ddiv_rn((double)val[0], (double)t.n));
+        if (stat) { stat[2 * blockIdx.x] = PYSP_KEY_NONE; stat[2 * blockIdx.x + 1] = 0; }
+    }
 }
 
 // work item of the two flat-field passes: four photosites of a row (two CFA sites, alternating)

@@ -10,7 +10,6 @@
 #include <algorithm>
 #include <atomic>
 #include <map>
-#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -607,106 +606,37 @@ int pysp_fuse_exposures(const float* const* brackets, int32_t n, int64_t in_pitc
 
 // ---- NumPy-ordered float32 plane sums (prepost.cuh) -----------------------------------------------------------------
 namespace {
-struct PlaneSumPlan {            // host layout of NumPy's pairwise-sum tree for n elements
-    std::vector<int> leaf_off, leaf_len, node_l, node_r, group_start;
-    std::vector<int> packed;     // the five tables back to back, as they are uploaded into the caller's workspace
-};
-
-int build_sum_tree(long long off, long long n, PlaneSumPlan& pl, std::vector<int>& height, std::vector<int>& h_of_val) {
-    // returns the value index of the subtree's result: leaves are (index), nodes are encoded as -(k+1) until renumbered
-    if (n <= 128) {
-        pl.leaf_off.push_back((int)off); pl.leaf_len.push_back((int)n);
-        return (int)pl.leaf_off.size() - 1;
-    }
-    long long n2 = n / 2;
-    n2 -= n2 % 8;
-    const int l = build_sum_tree(off, n2, pl, height, h_of_val);
-    const int r = build_sum_tree(off + n2, n - n2, pl, height, h_of_val);
-    auto h = [&](int v) { return v >= 0 ? 0 : height[-v - 1]; };
-    pl.node_l.push_back(l); pl.node_r.push_back(r);
-    height.push_back(std::max(h(l), h(r)) + 1);
-    return -(int)pl.node_l.size();
-}
-
-std::shared_ptr<const PlaneSumPlan> plane_sum_plan(long long n) {
-    // host-side cache of the last few plane sizes (bounded: the oldest entry is dropped); plans are immutable and shared
-    static std::mutex mu;
-    static std::vector<std::pair<long long, std::shared_ptr<const PlaneSumPlan>>> cache;
-    std::lock_guard<std::mutex> lk(mu);
-    for (auto& e : cache)
-        if (e.first == n) return e.second;
-    auto pl = std::make_shared<PlaneSumPlan>();
-    std::vector<int> height, unused;
-    build_sum_tree(0, n, *pl, height, unused);
-    const int nn = (int)pl->node_l.size(), nl = (int)pl->leaf_off.size();
-    std::vector<int> order(nn), rank(nn);
-    for (int k = 0; k < nn; ++k) order[k] = k;
-    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return height[a] < height[b]; });
-    for (int k = 0; k < nn; ++k) rank[order[k]] = k;
-    std::vector<int> nl_(nn), nr_(nn);
-    auto val = [&](int v) { return v >= 0 ? v : nl + rank[-v - 1]; };
-    for (int k = 0; k < nn; ++k) { nl_[k] = val(pl->node_l[order[k]]); nr_[k] = val(pl->node_r[order[k]]); }
-    pl->node_l.swap(nl_); pl->node_r.swap(nr_);
-    pl->group_start.push_back(0);
-    for (int k = 1; k <= nn; ++k)
-        if (k == nn || height[order[k]] != height[order[k - 1]]) pl->group_start.push_back(k);
-    pl->packed.reserve(2 * (size_t)nl + 2 * (size_t)nn + pl->group_start.size());
-    pl->packed.insert(pl->packed.end(), pl->leaf_off.begin(), pl->leaf_off.end());
-    pl->packed.insert(pl->packed.end(), pl->leaf_len.begin(), pl->leaf_len.end());
-    pl->packed.insert(pl->packed.end(), pl->node_l.begin(), pl->node_l.end());
-    pl->packed.insert(pl->packed.end(), pl->node_r.begin(), pl->node_r.end());
-    pl->packed.insert(pl->packed.end(), pl->group_start.begin(), pl->group_start.end());
-    if (cache.size() >= 8) cache.erase(cache.begin());
-    cache.emplace_back(n, pl);
-    return pl;
-}
-
 long long align16(long long v) { return (v + 15) / 16 * 16; }
 
-struct FlatWorkspace { long long off_tab, off_val, off_mean, off_stat, total; };
+struct FlatWorkspace { long long off_val, off_mean, off_stat, total; };
 
-FlatWorkspace flat_workspace_layout(const PlaneSumPlan& pl) {
+// the workspace depends on the plane's element count n alone: the tree's values (heap order, four planes), mean[4], stat[8]
+FlatWorkspace flat_workspace_layout(long long n) {
     FlatWorkspace w;
     long long o = 0;
-    const long long nl = (long long)pl.leaf_off.size(), nn = (long long)pl.node_l.size();
-    w.off_tab = o; o = align16(o + 4 * (long long)pl.packed.size());
-    w.off_val = o; o = align16(o + 4 * 4 * (nl + nn));
+    w.off_val = o; o = align16(o + 4 * 4 * ((2LL << plane_sum_tree(n, nullptr).L) - 1));
     w.off_mean = o; o = align16(o + 16);
     w.off_stat = o; o = align16(o + 32);
     w.total = o;
     return w;
 }
 
-// the tree tables are uploaded into the caller's workspace on the caller's stream (the library allocates nothing), then the
-// two summation kernels; mean[4] lands at ws + off_mean.  The host tables are pageable memory: cudaMemcpyAsync stages
-// them before it returns, so the plan may be evicted from the host cache afterwards.
-int launch_plane_means(const float* mosaic, long long pitch, int H, int W, char* ws, const PlaneSumPlan& pl, const FlatWorkspace& lay,
-                       PlaneSumTables* tables, cudaStream_t stream) {
-    const int nl = (int)pl.leaf_off.size(), nn = (int)pl.node_l.size(), ng = (int)pl.group_start.size() - 1;
-    int* d = (int*)(ws + lay.off_tab);
-    {
-        cudaError_t e = cudaMemcpyAsync(d, pl.packed.data(), pl.packed.size() * 4, cudaMemcpyHostToDevice, stream);
-        if (e != cudaSuccess) return fail(PYSP_ERR_CUDA, "plane means: table upload: %s", cudaGetErrorString(e));
-    }
-    PlaneSumTables t;
-    t.leaf_off = d; t.leaf_len = d + nl; t.node_l = d + 2 * nl; t.node_r = d + 2 * nl + nn; t.group_start = d + 2 * nl + 2 * nn;
-    t.n_leaves = nl; t.n_nodes = nn; t.n_groups = ng;
-    t.val = (float*)(ws + lay.off_val);
-    *tables = t;
-    leaf_sum_kernel<<<grid_for(32LL * nl, 256), 256, 0, stream>>>(mosaic, pitch, W, t);   // eight lanes per (plane, leaf)
+// the summation kernels on the caller's stream; mean[4] lands at `mean`.  With `stat`, tree_sum_kernel also resets the
+// flat-field statistics words.
+int launch_plane_means(const float* mosaic, long long pitch, int H, int W, char* ws, const FlatWorkspace& lay, float* mean,
+                       int* stat, cudaStream_t stream) {
+    const PlaneSumTree t = plane_sum_tree((long long)(H / 2) * (W / 2), (float*)(ws + lay.off_val));
+    leaf_sum_kernel<<<grid_for(32LL << t.L, 256), 256, 0, stream>>>(mosaic, pitch, W, t);   // eight lanes per (plane, node)
     int rc = check_launch("leaf_sum_kernel");
     if (rc) return rc;
-    const long long n = (long long)(H / 2) * (W / 2);
-    // wide levels of the tree run on the whole GPU, the narrow top of the tree in one block per plane
-    int g0 = 0;
-    for (; g0 < ng; ++g0) {
-        const int a = pl.group_start[g0], b = pl.group_start[g0 + 1];
-        if (b - a < 4096) break;
-        tree_level_kernel<<<dim3((unsigned)((b - a + 255) / 256), 4), 256, 0, stream>>>(t, a, b);
+    // wide levels of the tree (4096 nodes and more) run on the whole GPU, the narrow top of the tree in one block per plane
+    int d = t.L - 1;
+    for (; d >= 12; --d) {
+        tree_level_kernel<<<dim3((1u << d) / 256, 4), 256, 0, stream>>>(t, d);
         rc = check_launch("tree_level_kernel");
         if (rc) return rc;
     }
-    tree_sum_kernel<<<4, 1024, 0, stream>>>(t, g0, n, (float*)(ws + lay.off_mean));
+    tree_sum_kernel<<<4, 1024, 0, stream>>>(t, d, mean, stat);
     return check_launch("tree_sum_kernel");
 }
 }  // namespace
@@ -715,8 +645,7 @@ extern "C" {
 
 int64_t pysp_flat_workspace_bytes(int32_t H, int32_t W) {
     if (H < 2 || W < 2 || (H & 1) || (W & 1)) return 0;
-    auto pl = plane_sum_plan((long long)(H / 2) * (W / 2));
-    return flat_workspace_layout(*pl).total;
+    return flat_workspace_layout((long long)(H / 2) * (W / 2)).total;
 }
 
 int pysp_bayer_plane_means(const float* mosaic, int64_t pitch, int32_t H, int32_t W, float* means, void* workspace,
@@ -727,15 +656,9 @@ int pysp_bayer_plane_means(const float* mosaic, int64_t pitch, int32_t H, int32_
     if (pitch < 4LL * W) return fail(PYSP_ERR_INVALID, "pysp_bayer_plane_means: bad pitch");
     int rc = ensure_device();
     if (rc) return rc;
-    auto pl = plane_sum_plan((long long)(H / 2) * (W / 2));
-    const FlatWorkspace lay = flat_workspace_layout(*pl);
+    const FlatWorkspace lay = flat_workspace_layout((long long)(H / 2) * (W / 2));
     if (workspace_bytes < lay.total) return fail(PYSP_ERR_INVALID, "pysp_bayer_plane_means: workspace too small (%lld < %lld)", (long long)workspace_bytes, lay.total);
-    PlaneSumTables t;
-    rc = launch_plane_means(mosaic, pitch, H, W, (char*)workspace, *pl, lay, &t, stream);
-    if (rc) return rc;
-    cudaError_t e = cudaMemcpyAsync(means, (char*)workspace + lay.off_mean, 16, cudaMemcpyDeviceToDevice, stream);
-    if (e != cudaSuccess) return fail(PYSP_ERR_CUDA, "pysp_bayer_plane_means: %s", cudaGetErrorString(e));
-    return PYSP_OK;
+    return launch_plane_means(mosaic, pitch, H, W, (char*)workspace, lay, means, nullptr, stream);
 }
 
 int pysp_flat_frame_correction(const float* sensor, int64_t sensor_pitch, const float* flat, int64_t flat_pitch, float* out,
@@ -747,19 +670,15 @@ int pysp_flat_frame_correction(const float* sensor, int64_t sensor_pitch, const 
     if (sensor_pitch < 4LL * W || flat_pitch < 4LL * W || out_pitch < 4LL * W) return fail(PYSP_ERR_INVALID, "pysp_flat_frame_correction: bad pitch");
     int rc = ensure_device();
     if (rc) return rc;
-    auto pl = plane_sum_plan((long long)(H / 2) * (W / 2));
-    const FlatWorkspace lay = flat_workspace_layout(*pl);
+    const FlatWorkspace lay = flat_workspace_layout((long long)(H / 2) * (W / 2));
     if (workspace_bytes < lay.total) return fail(PYSP_ERR_INVALID, "pysp_flat_frame_correction: workspace too small (%lld < %lld)", (long long)workspace_bytes, lay.total);
     char* ws = (char*)workspace;
     FlatParams p;
-    rc = launch_plane_means(flat, flat_pitch, H, W, ws, *pl, lay, &p.t, stream);
-    if (rc) return rc;
-    const int stat0[8] = {PYSP_KEY_NONE, 0, PYSP_KEY_NONE, 0, PYSP_KEY_NONE, 0, PYSP_KEY_NONE, 0};
-    cudaError_t e = cudaMemcpyAsync(ws + lay.off_stat, stat0, sizeof(stat0), cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) return fail(PYSP_ERR_CUDA, "pysp_flat_frame_correction: %s", cudaGetErrorString(e));
     p.sensor = sensor; p.sensor_pitch = sensor_pitch; p.flat = flat; p.flat_pitch = flat_pitch; p.out = out; p.out_pitch = out_pitch;
     p.H = H; p.W = W; p.clamp_high = clamp_high;
     p.mean = (float*)(ws + lay.off_mean); p.stat = (int*)(ws + lay.off_stat);
+    rc = launch_plane_means(flat, flat_pitch, H, W, ws, lay, p.mean, p.stat, stream);
+    if (rc) return rc;
     flat_stats_kernel<<<grid_for((long long)H * W, 256), 256, 0, stream>>>(p);
     rc = check_launch("flat_stats_kernel");
     if (rc) return rc;

@@ -18,6 +18,7 @@ struct uint4 { unsigned int x, y, z, w; };
 #include "../../pysp_b200/csrc/eag.cuh"
 #include "../../pysp_b200/csrc/median_stage.cuh"
 #include "../../pysp_b200/csrc/develop_plan.h"
+#include "../../pysp_b200/csrc/prepost.cuh"
 
 using namespace pysp;
 
@@ -71,6 +72,29 @@ static void run_chain(const DevelopPlan& plan) {
             store_tile_generic<TW2, TH2>((const float*)(smem + LM::OFF_OUT), p.st, p.g, tx * TW2, p.y_begin + ty * TH2);
         }
     }
+}
+
+// NumPy's pairwise-sum tree of an n-element plane as leaf_sum_kernel walks it (prepost.cuh): one row (depth, index, first
+// element, count) per leaf, from left to right, and the level L of the kernel's work items in *L.  Returns the number of
+// leaves, or -1 when there are more than `cap`.
+extern "C" int emu_plane_sum_leaves(long long n, int* L, int64_t* rows, int cap) {
+    const PlaneSumTree t = plane_sum_tree(n, nullptr);
+    *L = t.L;
+    int k = 0;
+    auto leaf = [&](int d, int i, int first, int count) {
+        if (k == cap) return false;
+        int64_t* r = rows + 4 * (long long)k++;
+        r[0] = d; r[1] = i; r[2] = first; r[3] = count;
+        return true;
+    };
+    for (int i = 0; i < (1 << t.L); ++i) {
+        const SumNode e = sum_node(t, t.L, i);
+        const int l = leaf_part(e);
+        const bool ok = l == e.count ? leaf(t.L, i, e.first, l)
+                                     : leaf(t.L + 1, 2 * i, e.first, l) && leaf(t.L + 1, 2 * i + 1, e.first + l, e.count - l);
+        if (!ok) return -1;
+    }
+    return k;
 }
 
 extern "C" int emu_develop(const pysp_develop_args* a, int tw, int th) {

@@ -65,6 +65,38 @@ def test_flat_frame_correction_24mp(eng):
     assert_same_float_bits(got, ax.flat_frame_correction(sensor, flat), "24 MP flat-field correction")
 
 
+def test_plane_means_and_flat_field_are_graph_capturable(eng):
+    """include/pysp_b200.h: pysp_bayer_plane_means and pysp_flat_frame_correction only launch kernels (the summation tree
+    is derived on the device, the flat-field statistics are reset there), so both can be captured into one CUDA graph and
+    replayed on new inputs.  2050 x 2050: 1025^2 sites, leaves on two depths and a wide tree level; the flat fields
+    have zeros (+inf quotients replaced by the plane's maximum) and different maxima, so statistics left over from the
+    previous replay would show."""
+    H, W = 2050, 2050
+    rng = np.random.default_rng(9)
+    sens, flats = [], []
+    for k in range(2):
+        sens.append(eng.to_device(rng.random((H, W), dtype=np.float32)))
+        f = (0.5 + (1.5 - k) * rng.random((H, W), dtype=np.float32)).astype(np.float32)
+        f[rng.integers(0, H, 40), rng.integers(0, W, 40)] = 0.0
+        flats.append(eng.to_device(f))
+    want = [(eng.bayer_plane_means(f), eng.flat_frame_correction(s, f)) for s, f in zip(sens, flats)]
+    src_s, src_f = sens[0].clone(), flats[0].clone()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        means = eng.bayer_plane_means(src_f)
+        out = eng.flat_frame_correction(src_s, src_f)
+    for k in range(2):
+        src_s.copy_(sens[k])                # new inputs in the captured buffers, same graph
+        src_f.copy_(flats[k])
+        means.zero_()
+        out.zero_()
+        g.replay()
+        torch.cuda.synchronize()
+        assert torch.equal(means.view(torch.int32), want[k][0].view(torch.int32)), k
+        assert torch.equal(out.view(torch.int32), want[k][1].view(torch.int32)), k
+
+
 @pytest.mark.parametrize("name", HOT)
 def test_hot_pixels_fixtures(eng, name):
     from pysp_b200 import find_erroneous_pixels_threshold
