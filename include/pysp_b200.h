@@ -240,7 +240,8 @@ int pysp_warp_rectilinear_apply(const float* src, float* dst, int32_t height, in
  *     Image.merge("YCbCr", [Y, upsample2x2(Cb), upsample2x2(Cr)]).save(f, "JPEG", quality=quality, subsampling=2)
  * When W is a multiple of 16 and the planes are PYSP_OUT_YCC420_U8 of a develop, that is also byte-identical to the JPEG
  * libjpeg writes from the PYSP_OUT_SRGB_U8 image of the same call (for other widths libjpeg pads the chroma's right edge from
- * full-resolution chroma, which the planes do not hold).  What it does, all in integers (tests/jpeg_ref.py restates it):
+ * full-resolution chroma, which the planes do not hold; pysp_jpeg_encode_rgb below encodes the RGB image at any size).  What
+ * it does, all in integers (tests/jpeg_ref.py restates it):
  *  - markers SOI, APP0 (JFIF 1.01, density 1:1, no units), DQT luma, DQT chroma (8-bit, zigzag order), SOF0, DHT DC0, AC0,
  *    DC1, AC1 (the standard tables of Annex K.3), SOS, the entropy-coded data, EOI; MCU = Y00 Y01 Y10 Y11 Cb Cr, no restarts;
  *  - quantisation tables: scale = quality < 50 ? 5000/quality : 200 - 2*quality, clamp((std*scale + 50)/100, 1, 255) on
@@ -268,6 +269,41 @@ int64_t pysp_jpeg_workspace_bytes(int32_t height, int32_t width);
 int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t chroma_pitch,
                             int32_t height, int32_t width, int32_t quality, uint8_t* out, int64_t out_capacity,
                             int64_t* out_len, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---- baseline JPEG of an 8-bit RGB image at 4:4:4, 4:2:2 or 4:2:0 ------------------------------------------------------
+ *
+ * pysp_jpeg_encode_rgb writes one complete JFIF file byte-identical to libjpeg(-turbo)'s encode of the image with its
+ * defaults, i.e. Pillow's
+ *     Image.fromarray(S, "RGB").save(f, "JPEG", quality=quality, subsampling=subsampling)
+ * for any height and width.  `subsampling` takes Pillow's integers: */
+#define PYSP_JPEG_444 0    /* Y sampled 1x1: an MCU is Y Cb Cr */
+#define PYSP_JPEG_422 1    /* Y 2x1: Y0 Y1 Cb Cr */
+#define PYSP_JPEG_420 2    /* Y 2x2: Y00 Y01 Y10 Y11 Cb Cr */
+/* With (h, v) the Y sampling factors, MCUs mx = ceil(W / 8h) across and my = ceil(H / 8v) down, all in integers
+ * (tests/jpeg_rgb_ref.py restates it):
+ *  - colour: Y, cb, cr of every pixel as PYSP_OUT_YCC420_U8 states it (jccolor.c rgb_ycc_convert);
+ *  - chroma (jcsample.c): cb / cr with the last column repeated out to 8h * mx columns and the last row out to a multiple of v
+ *    rows, then downsampled: 4:4:4 a copy, 4:2:2 (a + b + bias) >> 1 with bias 0, 1, 0, 1, ... along the row, 4:2:0 the
+ *    2x2 average of PYSP_OUT_YCC420_U8 (bias 1, 2, 1, 2, ...); the last downsampled row is repeated out to 8 * my rows.
+ *    Repeating after the downsample instead is not the same: that is why planes developed at 4:2:0 give libjpeg's file of the
+ *    RGB image only when W % 16 == 0, and why this entry point takes the RGB image;
+ *  - Y: padded to whole blocks by repeating its last column and row; an MCU holds h x v Y slots in raster order, then Cb, Cr;
+ *    a Y slot outside the Y blocks is a dummy (AC zero, DC = the DC of the slot before it);
+ *  - header: that of pysp_jpeg_encode_ycc420 with the Y sampling byte of SOF0 set to (h << 4) | v; the rest (tables, DCT,
+ *    quantisation, Huffman coding, padding, stuffing) is the same.
+ * rgb: [height][width][3] R, G, B bytes, row pitch pitch_bytes >= 3 * width, any alignment; height and width 1..65535;
+ * quality 1..100.  out: >= pysp_jpeg_rgb_max_bytes(height, width, subsampling) bytes (out_capacity); *out_len (a DEVICE
+ * int64) receives the file's length, and no byte of `out` past it is written.  workspace: >=
+ * pysp_jpeg_rgb_workspace_bytes(...) bytes (the converted planes live there).  As for pysp_jpeg_encode_ycc420: every argument
+ * is checked before any CUDA call, nothing is allocated, no host <-> device copy, no synchronise, capturable in a CUDA graph. */
+/* The worst case of the file: pysp_jpeg_max_bytes's derivation with h * v + 2 blocks of at most 1660 bits per MCU:
+ * 623 + 2 * ceil((h * v + 2) * mx * my * 1660 / 8) + 2 bytes.  0 for an invalid size or subsampling. */
+int64_t pysp_jpeg_rgb_max_bytes(int32_t height, int32_t width, int32_t subsampling);
+/* Bytes of device workspace pysp_jpeg_encode_rgb needs (0 for an invalid size or subsampling). */
+int64_t pysp_jpeg_rgb_workspace_bytes(int32_t height, int32_t width, int32_t subsampling);
+int pysp_jpeg_encode_rgb(const uint8_t* rgb, int64_t pitch_bytes, int32_t height, int32_t width, int32_t quality,
+                         int32_t subsampling, uint8_t* out, int64_t out_capacity, int64_t* out_len, void* workspace,
+                         int64_t workspace_bytes, void* stream);
 
 /* Bench instrumentation (no reference counterpart): when enabled, pysp_develop brackets each kernel launch
  * with CUDA events on the launching stream; collect() synchronises them and returns, per kernel slot

@@ -14,6 +14,7 @@ CFA = {"RGGB": 1, "BGGR": 2, "GRBG": 3, "GBRG": 4}
 IN_U16, IN_F32 = 0, 1
 OUT_CAM_F32, OUT_LIN_F32, OUT_LIN_F16, OUT_SRGB_U8, OUT_SRGB_U16, OUT_YCC420_U8 = 0, 1, 2, 3, 4, 5
 QUALITY_BEST, QUALITY_FAST = 0, 1
+JPEG_444, JPEG_422, JPEG_420 = 0, 1, 2
 MAX_BRACKETS = 16
 
 
@@ -109,6 +110,13 @@ def lib():
     L.pysp_jpeg_encode_ycc420.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
                                           C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     L.pysp_jpeg_encode_ycc420.restype = C.c_int
+    L.pysp_jpeg_rgb_max_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+    L.pysp_jpeg_rgb_max_bytes.restype = C.c_int64
+    L.pysp_jpeg_rgb_workspace_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+    L.pysp_jpeg_rgb_workspace_bytes.restype = C.c_int64
+    L.pysp_jpeg_encode_rgb.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64,
+                                       C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    L.pysp_jpeg_encode_rgb.restype = C.c_int
     L.pysp_timing_enable.argtypes = [C.c_int32]
     L.pysp_timing_enable.restype = None
     L.pysp_timing_collect.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int64)]

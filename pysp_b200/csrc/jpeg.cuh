@@ -1,11 +1,18 @@
-// pysp_b200 -- baseline JPEG encode of YCbCr 4:2:0 planes (pysp_jpeg_encode_ycc420), byte-identical to libjpeg-turbo's
-// encode of the same planes with its defaults (ISLOW DCT, Annex K quantisation and Huffman tables, no restart markers, JFIF
-// 1.01 header).  The contract is restated in NumPy by tests/jpeg_ref.py.
+// pysp_b200 -- baseline JPEG encode, byte-identical to libjpeg-turbo's encode with its defaults (ISLOW DCT, Annex K
+// quantisation and Huffman tables, no restart markers, JFIF 1.01 header), of YCbCr 4:2:0 planes (pysp_jpeg_encode_ycc420) or of
+// an 8-bit RGB image at 4:4:4, 4:2:2 or 4:2:0 (pysp_jpeg_encode_rgb).  The contracts are restated in NumPy by tests/jpeg_ref.py
+// and tests/jpeg_rgb_ref.py.
 //
-// Phases, each a kernel whose work items are independent (tests/host_emu/jpeg_emu.cpp runs them serially on the CPU):
+// An MCU holds h x v Y blocks (h, v = the luma sampling factors: 2x2 for 4:2:0, 2x1 for 4:2:2, 1x1 for 4:4:4), then one Cb and
+// one Cr block: `slots` = h*v + 2 blocks.  The chroma planes are read as planes of cw x ch samples.
+//
+// Phases, each a kernel whose work items are independent (tests/host_emu/jpeg_emu.cpp and jpeg_rgb_emu.cpp run them serially on
+// the CPU):
 //   header   one item per header byte (623 bytes: SOI APP0 DQT DQT SOF0 DHT x4 SOS) and per quantisation divisor;
-//   block    one item per 8x8 block in MCU order (Y00 Y01 Y10 Y11 Cb Cr): load with edge replication, ISLOW DCT, quantise,
-//            store the zigzag coefficients, and count the block's Huffman bits.  The DC predictor is the quantised DC of the
+//   convert  (RGB input only) one item per chroma sample: libjpeg's YCbCr of the h x v pixels it covers, the Y samples and the
+//            downsampled Cb / Cr stored as planes in the workspace; from there on the two entry points run the same phases;
+//   block    one item per 8x8 block in MCU order (Y slots in raster order, Cb, Cr): load with edge replication, ISLOW DCT,
+//            quantise, store the zigzag coefficients, and count the block's Huffman bits.  The DC predictor is the quantised DC of the
 //            block before it in the component; the ISLOW DC is exactly the sum of (x - 128) over the block, so it is
 //            recomputed from the pixels rather than waited for;
 //   scan     exclusive prefix sum of the block bit counts (64-bit offsets);
@@ -184,9 +191,13 @@ struct JpegParams {
     const uint8_t* cr;
     int64_t y_pitch, c_pitch;
     int H, W, quality;
+    int h, v;                  // Y blocks per MCU across / down (the luma sampling factors, 1 or 2; chroma is 1x1)
+    int slots;                 // blocks per MCU: h*v Y slots, Cb, Cr
+    uint32_t slots_m;          // jpeg_recip(slots): block b < 2^31 is in MCU jpeg_div(b, slots_m) (exact: m * slots - 2^32 <= 2)
+    int cw, ch;                // chroma plane width / height in samples
     int ybw, ybh;              // Y blocks across / down: ceil(W/8), ceil(H/8)
-    int mcux, mcuy;            // MCUs across / down: ceil(W/16), ceil(H/16) (= chroma blocks across / down)
-    int64_t n_blocks;          // 6 per MCU
+    int mcux, mcuy;            // MCUs across / down: ceil(W/8h), ceil(H/8v) (= chroma blocks across / down)
+    int64_t n_blocks;          // slots per MCU; below 2^31 for every size (at most 3 * 8192 * 8192 at 4:4:4)
     int64_t max_items;         // count / emit items of the largest possible stream
     uint8_t* out;
     int64_t* out_len;
@@ -201,13 +212,26 @@ struct JpegParams {
     uint32_t* ffcnt;           // [max_items] 0xFF bytes per item
     int64_t* foff;             // [max_items] 0xFF bytes before each item (exclusive scan of ffcnt)
     int64_t* fchunk;           // [ceil(max_items / JPEG_SCAN_CHUNK)] scan partials
+    // RGB input (pysp_jpeg_encode_rgb): the convert phase writes the planes y / cb / cr then read, in the workspace:
+    // Y [H][W], Cb and Cr [ch][cw] with cw = 8 * mcux, ch = ceil(H/v)
+    const uint8_t* rgb;        // [H][W][3], row pitch rgb_pitch bytes; nullptr for pysp_jpeg_encode_ycc420
+    int64_t rgb_pitch;
+    uint8_t* conv_y;
+    uint8_t* conv_cb;
+    uint8_t* conv_cr;
 };
+
+// luma sampling factors of Pillow's `subsampling` (PYSP_JPEG_444 / 422 / 420)
+static inline int jpeg_h(int subsampling) { return subsampling == 0 ? 1 : 2; }
+static inline int jpeg_v(int subsampling) { return subsampling == 2 ? 2 : 1; }
 
 static inline int64_t jpeg_align(int64_t v) { return (v + 255) / 256 * 256; }
 
-// The workspace layout; with base == nullptr only the size is computed.  Returns the total bytes.
-static inline int64_t jpeg_layout(int H, int W, char* base, JpegParams* p) {
-    const int64_t mcus = (int64_t)((W + 15) / 16) * ((H + 15) / 16), nb = 6 * mcus;
+// The workspace layout of an MCU of h x v Y blocks, plus the convert phase's planes when `planes`; with base == nullptr only the
+// size is computed.  Returns the total bytes.
+static inline int64_t jpeg_layout(int H, int W, int h, int v, bool planes, char* base, JpegParams* p) {
+    const int mcux = (W + 8 * h - 1) / (8 * h), mcuy = (H + 8 * v - 1) / (8 * v);
+    const int64_t mcus = (int64_t)mcux * mcuy, nb = (h * v + 2) * mcus;
     const int64_t max_bits = nb * JPEG_MAX_BLOCK_BITS;
     const int64_t max_items = ((max_bits + 7) / 8 + JPEG_EMIT_BYTES - 1) / JPEG_EMIT_BYTES;
     int64_t o = 0;
@@ -223,21 +247,45 @@ static inline int64_t jpeg_layout(int H, int W, char* base, JpegParams* p) {
     t.ffcnt = (uint32_t*)take(max_items * 4);
     t.foff = (int64_t*)take(max_items * 8);
     t.fchunk = (int64_t*)take((max_items + JPEG_SCAN_CHUNK - 1) / JPEG_SCAN_CHUNK * 8);
+    t.conv_y = t.conv_cb = t.conv_cr = nullptr;
+    if (planes) {
+        const int64_t nc = (int64_t)8 * mcux * ((H + v - 1) / v);
+        t.conv_y = (uint8_t*)take((int64_t)H * W);
+        t.conv_cb = (uint8_t*)take(nc);
+        t.conv_cr = (uint8_t*)take(nc);
+    }
     if (p) {
         p->qt = t.qt; p->totals = t.totals; p->coef = t.coef; p->bits = t.bits; p->boff = t.boff; p->bchunk = t.bchunk;
         p->words = t.words; p->ffcnt = t.ffcnt; p->foff = t.foff; p->fchunk = t.fchunk;
+        p->conv_y = t.conv_y; p->conv_cb = t.conv_cb; p->conv_cr = t.conv_cr;
         p->n_blocks = nb; p->max_items = max_items;
     }
     return o;
 }
 
-// Worst case of the file (see pysp_jpeg_max_bytes in include/pysp_b200.h)
-static inline int64_t jpeg_max_bytes(int H, int W) {
-    const int64_t nb = 6 * (int64_t)((W + 15) / 16) * ((H + 15) / 16);
+// the layout of pysp_jpeg_encode_ycc420 (4:2:0 planes)
+static inline int64_t jpeg_layout(int H, int W, char* base, JpegParams* p) { return jpeg_layout(H, W, 2, 2, false, base, p); }
+
+// Worst case of the file (see pysp_jpeg_max_bytes and pysp_jpeg_rgb_max_bytes in include/pysp_b200.h)
+static inline int64_t jpeg_max_bytes(int H, int W, int h, int v) {
+    const int64_t nb = (h * v + 2) * (int64_t)((W + 8 * h - 1) / (8 * h)) * ((H + 8 * v - 1) / (8 * v));
     return JPEG_HEADER_BYTES + 2 * ((nb * JPEG_MAX_BLOCK_BITS + 7) / 8) + 2;
 }
 
 static inline bool jpeg_size_ok(int H, int W) { return H >= 2 && W >= 2 && H <= 65535 && W <= 65535 && !(H & 1) && !(W & 1); }
+static inline bool jpeg_rgb_size_ok(int H, int W, int subsampling) {
+    return H >= 1 && W >= 1 && H <= 65535 && W <= 65535 && subsampling >= 0 && subsampling <= 2;
+}
+
+// geometry of an MCU of h x v Y blocks and cw x ch chroma planes
+static inline void jpeg_geometry(JpegParams* p, int H, int W, int h, int v, int cw, int ch, int quality, uint8_t* out,
+                                 int64_t* out_len) {
+    p->H = H; p->W = W; p->quality = quality;
+    p->h = h; p->v = v; p->slots = h * v + 2; p->slots_m = jpeg_recip(h * v + 2); p->cw = cw; p->ch = ch;
+    p->ybw = (W + 7) / 8; p->ybh = (H + 7) / 8; p->mcux = (W + 8 * h - 1) / (8 * h); p->mcuy = (H + 8 * v - 1) / (8 * v);
+    p->out = out; p->out_len = out_len;
+    p->rgb = nullptr; p->rgb_pitch = 0;
+}
 
 // Checks every argument before anything runs; fills *p.  err gets the reason of a PYSP_ERR_INVALID.
 static inline int plan_jpeg(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t c_pitch, int H, int W,
@@ -247,9 +295,9 @@ static inline int plan_jpeg(const uint8_t* y, int64_t y_pitch, const uint8_t* cb
     if (!jpeg_size_ok(H, W)) { snprintf(err, err_len, "pysp_jpeg_encode_ycc420: %dx%d: height and width must be even, 2..65535", H, W); return -1; }
     if (quality < 1 || quality > 100) { snprintf(err, err_len, "pysp_jpeg_encode_ycc420: quality %d outside 1..100", quality); return -1; }
     if (y_pitch < W || c_pitch < W / 2) { snprintf(err, err_len, "pysp_jpeg_encode_ycc420: pitch below the plane width"); return -1; }
-    if (out_capacity < jpeg_max_bytes(H, W)) {
+    if (out_capacity < jpeg_max_bytes(H, W, 2, 2)) {
         snprintf(err, err_len, "pysp_jpeg_encode_ycc420: out_capacity %lld < pysp_jpeg_max_bytes = %lld", (long long)out_capacity,
-                 (long long)jpeg_max_bytes(H, W));
+                 (long long)jpeg_max_bytes(H, W, 2, 2));
         return -1;
     }
     const int64_t need = jpeg_layout(H, W, nullptr, nullptr);
@@ -258,17 +306,47 @@ static inline int plan_jpeg(const uint8_t* y, int64_t y_pitch, const uint8_t* cb
         return -1;
     }
     jpeg_layout(H, W, (char*)ws, p);
+    jpeg_geometry(p, H, W, 2, 2, W / 2, H / 2, quality, out, out_len);
     p->y = y; p->cb = cb; p->cr = cr; p->y_pitch = y_pitch; p->c_pitch = c_pitch;
-    p->H = H; p->W = W; p->quality = quality;
-    p->ybw = (W + 7) / 8; p->ybh = (H + 7) / 8; p->mcux = (W + 15) / 16; p->mcuy = (H + 15) / 16;
-    p->out = out; p->out_len = out_len;
+    return 0;
+}
+
+// The same for pysp_jpeg_encode_rgb: the block phases read the convert phase's planes in the workspace.
+static inline int plan_jpeg_rgb(const uint8_t* rgb, int64_t pitch, int H, int W, int quality, int subsampling, uint8_t* out,
+                                int64_t out_capacity, int64_t* out_len, void* ws, int64_t ws_bytes, JpegParams* p, char* err,
+                                size_t err_len) {
+    if (!rgb || !out || !out_len || !ws) { snprintf(err, err_len, "pysp_jpeg_encode_rgb: null pointer"); return -1; }
+    if (subsampling < 0 || subsampling > 2) {
+        snprintf(err, err_len, "pysp_jpeg_encode_rgb: subsampling %d is not PYSP_JPEG_444 / 422 / 420 (0 / 1 / 2)", subsampling);
+        return -1;
+    }
+    if (!jpeg_rgb_size_ok(H, W, subsampling)) { snprintf(err, err_len, "pysp_jpeg_encode_rgb: %dx%d: height and width must be 1..65535", H, W); return -1; }
+    if (quality < 1 || quality > 100) { snprintf(err, err_len, "pysp_jpeg_encode_rgb: quality %d outside 1..100", quality); return -1; }
+    if (pitch < 3 * (int64_t)W) { snprintf(err, err_len, "pysp_jpeg_encode_rgb: pitch %lld below 3 * width", (long long)pitch); return -1; }
+    const int h = jpeg_h(subsampling), v = jpeg_v(subsampling);
+    if (out_capacity < jpeg_max_bytes(H, W, h, v)) {
+        snprintf(err, err_len, "pysp_jpeg_encode_rgb: out_capacity %lld < pysp_jpeg_rgb_max_bytes = %lld", (long long)out_capacity,
+                 (long long)jpeg_max_bytes(H, W, h, v));
+        return -1;
+    }
+    const int64_t need = jpeg_layout(H, W, h, v, true, nullptr, nullptr);
+    if (ws_bytes < need) {
+        snprintf(err, err_len, "pysp_jpeg_encode_rgb: workspace %lld < pysp_jpeg_rgb_workspace_bytes = %lld", (long long)ws_bytes,
+                 (long long)need);
+        return -1;
+    }
+    jpeg_layout(H, W, h, v, true, (char*)ws, p);
+    const int mcux = (W + 8 * h - 1) / (8 * h);
+    jpeg_geometry(p, H, W, h, v, 8 * mcux, (H + v - 1) / v, quality, out, out_len);
+    p->rgb = rgb; p->rgb_pitch = pitch;
+    p->y = p->conv_y; p->cb = p->conv_cb; p->cr = p->conv_cr; p->y_pitch = W; p->c_pitch = p->cw;
     return 0;
 }
 
 // ---- header ---------------------------------------------------------------------------------------------------------
 // byte i of SOI, APP0 (JFIF 1.01, no units, density 1:1), DQT luma, DQT chroma (8-bit, zigzag order), SOF0 (3 components,
-// Y 2x2, Cb and Cr 1x1), DHT DC0, AC0, DC1, AC1, SOS (Y: tables 0/0, Cb and Cr: 1/1, Ss 0, Se 63, Ah Al 0)
-PYSP_HD uint8_t jpeg_header_byte(int i, int H, int W, int quality) {
+// Y h x v (`hv` = h << 4 | v), Cb and Cr 1x1), DHT DC0, AC0, DC1, AC1, SOS (Y: tables 0/0, Cb and Cr: 1/1, Ss 0, Se 63, Ah Al 0)
+PYSP_HD uint8_t jpeg_header_byte(int i, int H, int W, int quality, int hv) {
     if (i < 20) {
         const uint8_t a[20] = {0xFF, 0xD8, 0xFF, 0xE0, 0, 16, 'J', 'F', 'I', 'F', 0, 1, 1, 0, 0, 1, 0, 1, 0, 0};
         return a[i];
@@ -280,8 +358,8 @@ PYSP_HD uint8_t jpeg_header_byte(int i, int H, int W, int quality) {
     }
     if (i < 177) {                                     // SOF0
         const uint8_t a[19] = {0xFF, 0xC0, 0, 17, 8, (uint8_t)(H >> 8), (uint8_t)H, (uint8_t)(W >> 8), (uint8_t)W, 3,
-                               1, 0x22, 0, 2, 0x11, 1, 3, 0x11, 1};
-        return a[i - 158];
+                               1, 0, 0, 2, 0x11, 1, 3, 0x11, 1};
+        return i == 169 ? (uint8_t)hv : a[i - 158];
     }
     if (i < 609) {                                     // DHT: DC (33 bytes), AC (183 bytes), DC, AC
         int j = i - 177, t = 0;
@@ -306,7 +384,7 @@ PYSP_HD uint8_t jpeg_header_byte(int i, int H, int W, int quality) {
 
 // header item i (i < JPEG_HEADER_BYTES) and divisor item i (i < 128)
 PYSP_HD void jpeg_header_item(const JpegParams& p, int i) {
-    if (i < JPEG_HEADER_BYTES) p.out[i] = jpeg_header_byte(i, p.H, p.W, p.quality);
+    if (i < JPEG_HEADER_BYTES) p.out[i] = jpeg_header_byte(i, p.H, p.W, p.quality, (p.h << 4) | p.v);
     if (i < 128) {
         const uint32_t d = 8u * (uint32_t)jpeg_quant_value(i >> 6, i & 63, p.quality);
         p.qt[i] = d;
@@ -314,19 +392,43 @@ PYSP_HD void jpeg_header_item(const JpegParams& p, int i) {
     }
 }
 
+// ---- conversion of RGB input ----------------------------------------------------------------------------------------
+// convert item (cx, cy), cx < cw, cy < ch: chroma sample (cx, cy) and the Y samples of the h x v pixels it covers
+// (jccolor.c rgb_ycc_convert, as PYSP_OUT_YCC420_U8 states it).  Full-resolution chroma is taken with the last column and row
+// of the image repeated past its edges, then downsampled (jcsample.c): 4:2:2 (a + b + (cx & 1)) >> 1 (h2v1_downsample),
+// 4:2:0 (a + b + c + d + 1 + (cx & 1)) >> 2 (h2v2_downsample), 4:4:4 a copy.  The block loader repeats the last chroma row.
+PYSP_HD void jpeg_convert_item(const JpegParams& p, int cx, int cy) {
+    int sb = 0, sr = 0;
+    for (int dy = 0; dy < p.v; ++dy) {
+        const int y = cy * p.v + dy, yy = y < p.H ? y : p.H - 1;
+        const uint8_t* row = p.rgb + yy * p.rgb_pitch;
+        for (int dx = 0; dx < p.h; ++dx) {
+            const int x = cx * p.h + dx, xx = x < p.W ? x : p.W - 1;
+            const int R = row[3 * xx], G = row[3 * xx + 1], B = row[3 * xx + 2];
+            if (x < p.W && y < p.H) p.conv_y[(int64_t)y * p.W + x] = (uint8_t)((19595 * R + 38470 * G + 7471 * B + 32768) >> 16);
+            sb += (-11059 * R - 21709 * G + 32768 * B + (128 << 16) + 32767) >> 16;
+            sr += (32768 * R - 27439 * G - 5329 * B + (128 << 16) + 32767) >> 16;
+        }
+    }
+    const int n = p.h * p.v, bias = n == 1 ? 0 : (cx & 1) + (n >> 2), sh = n >> 1;
+    const int64_t o = (int64_t)cy * p.cw + cx;
+    p.conv_cb[o] = (uint8_t)((sb + bias) >> sh);
+    p.conv_cr[o] = (uint8_t)((sr + bias) >> sh);
+}
+
 // ---- blocks ---------------------------------------------------------------------------------------------------------
 struct JpegBlock { const uint8_t* plane; int64_t pitch; int h, w, by, bx, comp; bool real; };
 
-// block b in MCU order: slots 0-3 are Y (2x2), 4 Cb, 5 Cr.  A Y slot outside the Y blocks is a dummy.
+// block b in MCU order: slots 0 .. h*v-1 are Y (h x v, raster order), then Cb, Cr.  A Y slot outside the Y blocks is a dummy.
 PYSP_HD JpegBlock jpeg_block_at(const JpegParams& p, int64_t mcu, int slot) {
     JpegBlock k;
-    const int my = (int)(mcu / p.mcux), mx = (int)(mcu - (int64_t)my * p.mcux);
-    if (slot < 4) {
+    const int my = (int)(mcu / p.mcux), mx = (int)(mcu - (int64_t)my * p.mcux), ny = p.slots - 2;
+    if (slot < ny) {
         k.plane = p.y; k.pitch = p.y_pitch; k.h = p.H; k.w = p.W; k.comp = 0;
-        k.by = 2 * my + (slot >> 1); k.bx = 2 * mx + (slot & 1);
+        k.by = p.v * my + (slot >> (p.h - 1)); k.bx = p.h * mx + (slot & (p.h - 1));     // h is 1 or 2
         k.real = k.by < p.ybh && k.bx < p.ybw;
     } else {
-        k.plane = slot == 4 ? p.cb : p.cr; k.pitch = p.c_pitch; k.h = p.H / 2; k.w = p.W / 2; k.comp = slot - 3;
+        k.plane = slot == ny ? p.cb : p.cr; k.pitch = p.c_pitch; k.h = p.ch; k.w = p.cw; k.comp = slot - ny + 1;
         k.by = my; k.bx = mx; k.real = true;
     }
     return k;
@@ -361,9 +463,10 @@ PYSP_HD int jpeg_slot_dc(const JpegParams& p, const uint32_t* qt, int64_t mcu, i
 
 // DC predictor of block b: the quantised DC of the previous block of the same component (0 for the first)
 PYSP_HD int jpeg_dc_pred(const JpegParams& p, const uint32_t* qt, int64_t mcu, int slot) {
-    if (slot >= 1 && slot <= 3) return jpeg_slot_dc(p, qt, mcu, slot - 1);
+    const int ny = p.slots - 2;
+    if (slot >= 1 && slot < ny) return jpeg_slot_dc(p, qt, mcu, slot - 1);
     if (mcu == 0) return 0;
-    return jpeg_slot_dc(p, qt, mcu - 1, slot == 0 ? 3 : slot);
+    return jpeg_slot_dc(p, qt, mcu - 1, slot == 0 ? ny - 1 : slot);
 }
 
 #define PYSP_DESCALE(x, n) (((x) + (1 << ((n) - 1))) >> (n))
@@ -424,8 +527,8 @@ struct JpegBitCount {
 
 // block item: DCT, quantisation, zigzag store, bit count.  qt / huff may be shared-memory copies.
 PYSP_HD void jpeg_block_item(const JpegParams& p, const uint32_t* qt, const uint32_t* huff, int64_t b) {
-    const int64_t mcu = b / 6;
-    const int slot = (int)(b - 6 * mcu);
+    const int64_t mcu = jpeg_div((uint32_t)b, p.slots_m);          // b < n_blocks < 2^31
+    const int slot = (int)(b - p.slots * mcu);
     const JpegBlock k = jpeg_block_at(p, mcu, slot);
     const int t = k.comp ? 64 : 0;
     int zz[64];
@@ -491,9 +594,9 @@ struct JpegBitWriter {
 
 // pack item: block b's codes at its bit offset (the zero phase has cleared the words first)
 PYSP_HD void jpeg_pack_item(const JpegParams& p, const uint32_t* huff, int64_t b) {
-    const int64_t mcu = b / 6;
-    const int slot = (int)(b - 6 * mcu);
-    const int comp = slot < 4 ? 0 : slot - 3;
+    const int64_t mcu = jpeg_div((uint32_t)b, p.slots_m);          // b < n_blocks < 2^31
+    const int slot = (int)(b - p.slots * mcu), ny = p.slots - 2;
+    const int comp = slot < ny ? 0 : slot - ny + 1;
     int zz[64];
     const uint32_t* src = (const uint32_t*)(p.coef + 64 * b);
 #pragma unroll
@@ -504,8 +607,8 @@ PYSP_HD void jpeg_pack_item(const JpegParams& p, const uint32_t* huff, int64_t b
     }
     // DC of the previous block of the component, from the stored coefficients
     int pred = 0;
-    if (slot >= 1 && slot <= 3) pred = p.coef[64 * (b - 1)];
-    else if (mcu > 0) pred = p.coef[64 * (slot == 0 ? b - 3 : b - 6)];
+    if (slot >= 1 && slot < ny) pred = p.coef[64 * (b - 1)];
+    else if (mcu > 0) pred = p.coef[64 * (slot == 0 ? b - 3 : b - p.slots)];      // slot 0: the last Y slot, 3 blocks back
     const int64_t pos = p.boff[b];
     JpegBitWriter wr;
     wr.words = p.words; wr.w = pos >> 5; wr.acc = 0; wr.nacc = (int)(pos & 31); wr.first = true;
@@ -560,6 +663,12 @@ constexpr int JPEG_SCAN_PER = JPEG_SCAN_CHUNK / JPEG_THREADS;
 
 __global__ void __launch_bounds__(JPEG_THREADS) jpeg_header_kernel(const JpegParams p) {
     for (int i = threadIdx.x; i < JPEG_HEADER_BYTES; i += blockDim.x) jpeg_header_item(p, i);
+}
+
+// one row of chroma samples per blockIdx.y
+__global__ void __launch_bounds__(JPEG_THREADS) jpeg_convert_kernel(const JpegParams p) {
+    const int cx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (cx < p.cw) jpeg_convert_item(p, cx, blockIdx.y);
 }
 
 __device__ __forceinline__ void jpeg_tables_to_smem(uint32_t* s_huff, uint32_t* s_qt, const uint32_t* qt) {

@@ -805,23 +805,10 @@ int pysp_warp_rectilinear_apply(const float* src, float* dst, int32_t H, int32_t
 
 }  // extern "C"
 
-// ---- baseline JPEG of YCbCr 4:2:0 planes (jpeg.cuh) ------------------------------------------------------------------
-extern "C" {
-
-int64_t pysp_jpeg_max_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_max_bytes(H, W) : 0; }
-
-int64_t pysp_jpeg_workspace_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_layout(H, W, nullptr, nullptr) : 0; }
-
-int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t chroma_pitch, int32_t H,
-                            int32_t W, int32_t quality, uint8_t* out, int64_t out_capacity, int64_t* out_len, void* workspace,
-                            int64_t workspace_bytes, void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
-    JpegParams p;
-    if (plan_jpeg(y, y_pitch, cb, cr, chroma_pitch, H, W, quality, out, out_capacity, out_len, workspace, workspace_bytes, &p, g_err,
-                  sizeof(g_err)))
-        return PYSP_ERR_INVALID;
-    int rc = ensure_device();
-    if (rc) return rc;
+// ---- baseline JPEG of YCbCr 4:2:0 planes or of RGB images (jpeg.cuh) ---------------------------------------------------
+// the phases of one encode, in order; the convert phase only for RGB input
+static int jpeg_launch(const JpegParams& p, cudaStream_t stream) {
+    int rc;
     const long long cap = 148LL * 8;                     // fixed grids of the kernels whose item count is on the device
     const int block_grid = (int)((p.n_blocks + JPEG_THREADS - 1) / JPEG_THREADS);
     const long long bchunks = (p.n_blocks + JPEG_SCAN_CHUNK - 1) / JPEG_SCAN_CHUNK;
@@ -830,6 +817,10 @@ int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb
     const JpegScan fscan = {p.ffcnt, p.foff, p.fchunk, p.totals + 1, 0, p.totals};
     jpeg_header_kernel<<<1, JPEG_THREADS, 0, stream>>>(p);
     if ((rc = check_launch("jpeg_header_kernel"))) return rc;
+    if (p.rgb) {
+        jpeg_convert_kernel<<<dim3((p.cw + JPEG_THREADS - 1) / JPEG_THREADS, p.ch), JPEG_THREADS, 0, stream>>>(p);
+        if ((rc = check_launch("jpeg_convert_kernel"))) return rc;
+    }
     jpeg_block_kernel<<<block_grid, JPEG_THREADS, 0, stream>>>(p);
     if ((rc = check_launch("jpeg_block_kernel"))) return rc;
     jpeg_scan_reduce_kernel<<<(int)std::min(bchunks, cap), JPEG_THREADS, 0, stream>>>(bscan);
@@ -852,6 +843,44 @@ int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb
     if ((rc = check_launch("jpeg_scan_down_kernel"))) return rc;
     jpeg_emit_kernel<<<(int)cap, JPEG_THREADS, 0, stream>>>(p);
     return check_launch("jpeg_emit_kernel");
+}
+
+extern "C" {
+
+int64_t pysp_jpeg_max_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_max_bytes(H, W, 2, 2) : 0; }
+
+int64_t pysp_jpeg_workspace_bytes(int32_t H, int32_t W) { return jpeg_size_ok(H, W) ? jpeg_layout(H, W, nullptr, nullptr) : 0; }
+
+int pysp_jpeg_encode_ycc420(const uint8_t* y, int64_t y_pitch, const uint8_t* cb, const uint8_t* cr, int64_t chroma_pitch, int32_t H,
+                            int32_t W, int32_t quality, uint8_t* out, int64_t out_capacity, int64_t* out_len, void* workspace,
+                            int64_t workspace_bytes, void* stream) {
+    JpegParams p;
+    if (plan_jpeg(y, y_pitch, cb, cr, chroma_pitch, H, W, quality, out, out_capacity, out_len, workspace, workspace_bytes, &p, g_err,
+                  sizeof(g_err)))
+        return PYSP_ERR_INVALID;
+    int rc = ensure_device();
+    if (rc) return rc;
+    return jpeg_launch(p, (cudaStream_t)stream);
+}
+
+int64_t pysp_jpeg_rgb_max_bytes(int32_t H, int32_t W, int32_t subsampling) {
+    return jpeg_rgb_size_ok(H, W, subsampling) ? jpeg_max_bytes(H, W, jpeg_h(subsampling), jpeg_v(subsampling)) : 0;
+}
+
+int64_t pysp_jpeg_rgb_workspace_bytes(int32_t H, int32_t W, int32_t subsampling) {
+    return jpeg_rgb_size_ok(H, W, subsampling) ? jpeg_layout(H, W, jpeg_h(subsampling), jpeg_v(subsampling), true, nullptr, nullptr)
+                                               : 0;
+}
+
+int pysp_jpeg_encode_rgb(const uint8_t* rgb, int64_t pitch_bytes, int32_t H, int32_t W, int32_t quality, int32_t subsampling,
+                         uint8_t* out, int64_t out_capacity, int64_t* out_len, void* workspace, int64_t workspace_bytes, void* stream) {
+    JpegParams p;
+    if (plan_jpeg_rgb(rgb, pitch_bytes, H, W, quality, subsampling, out, out_capacity, out_len, workspace, workspace_bytes, &p, g_err,
+                      sizeof(g_err)))
+        return PYSP_ERR_INVALID;
+    int rc = ensure_device();
+    if (rc) return rc;
+    return jpeg_launch(p, (cudaStream_t)stream);
 }
 
 }  // extern "C"

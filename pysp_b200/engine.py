@@ -281,6 +281,64 @@ def encode_jpeg(planes, quality=75, out_tensor=None, stream=None):
     return out_tensor, n
 
 
+_SUBSAMPLINGS = {"4:4:4": _capi.JPEG_444, "4:2:2": _capi.JPEG_422, "4:2:0": _capi.JPEG_420,
+                 0: _capi.JPEG_444, 1: _capi.JPEG_422, 2: _capi.JPEG_420}
+
+
+def jpeg_subsampling(subsampling):
+    """PYSP_JPEG_444 / 422 / 420 of "4:4:4" / "4:2:2" / "4:2:0" or Pillow's integers 0 / 1 / 2"""
+    s = _SUBSAMPLINGS.get(subsampling) if isinstance(subsampling, (str, int)) and not isinstance(subsampling, bool) else None
+    if s is None:
+        raise ValueError('JPEG subsampling must be "4:4:4", "4:2:2", "4:2:0" or 0, 1, 2 (got %r)' % (subsampling,))
+    return s
+
+
+def jpeg_rgb_max_bytes(height, width, subsampling="4:2:0"):
+    """pysp_jpeg_rgb_max_bytes: the largest file encode_jpeg_rgb can write for an H x W image"""
+    n = int(_capi.lib().pysp_jpeg_rgb_max_bytes(int(height), int(width), jpeg_subsampling(subsampling)))
+    if n <= 0:
+        raise ValueError("jpeg_rgb_max_bytes: height and width must be 1..65535 (got %dx%d)" % (height, width))
+    return n
+
+
+def encode_jpeg_rgb(rgb, quality=75, subsampling="4:2:0", out_tensor=None, stream=None):
+    """Baseline JPEG of an 8-bit RGB image on the device (include/pysp_b200.h, pysp_jpeg_encode_rgb): byte-identical to
+    libjpeg's encode of the image at any size (Pillow: Image.fromarray(S, "RGB").save(f, "JPEG", quality=quality,
+    subsampling=subsampling)).
+
+    rgb          uint8 CUDA tensor [H, W, 3] with strides (pitch, 3, 1), any pitch >= 3W, e.g. what develop(out="srgb_u8")
+                 returns; H and W 1..65535.
+    subsampling  "4:4:4" / "4:2:2" / "4:2:0", or Pillow's 0 / 1 / 2.
+    out_tensor   optional flat uint8 CUDA tensor of >= jpeg_rgb_max_bytes(H, W, subsampling) bytes.
+    Returns (buf, n) as encode_jpeg does: the file is the first n bytes of `buf`, `n` a 0-d int64 CUDA tensor, nothing is
+    synchronised.
+    """
+    require_cuda()
+    L = _capi.lib()
+    s = jpeg_subsampling(subsampling)
+    if not 1 <= int(quality) <= 100:
+        raise ValueError("encode_jpeg_rgb: quality %d outside 1..100" % int(quality))
+    if not (isinstance(rgb, torch.Tensor) and rgb.is_cuda and rgb.dtype == torch.uint8 and rgb.dim() == 3 and rgb.shape[2] == 3
+            and rgb.stride(2) == 1 and rgb.stride(1) == 3 and rgb.stride(0) >= 3 * rgb.shape[1]):
+        raise ValueError("encode_jpeg_rgb: rgb must be a uint8 CUDA tensor [H, W, 3] with strides (pitch >= 3W, 3, 1)")
+    H, W = int(rgb.shape[0]), int(rgb.shape[1])
+    dev = rgb.device
+    cap = jpeg_rgb_max_bytes(H, W, s)
+    with _on(dev, stream):
+        if out_tensor is None:
+            out_tensor = torch.empty(cap, dtype=torch.uint8, device=dev)
+        elif (not isinstance(out_tensor, torch.Tensor) or not out_tensor.is_cuda or out_tensor.dtype != torch.uint8
+              or out_tensor.dim() != 1 or not out_tensor.is_contiguous() or out_tensor.device != dev or out_tensor.numel() < cap):
+            raise ValueError("encode_jpeg_rgb: out_tensor must be a flat contiguous uint8 CUDA tensor of >= %d bytes on the "
+                             "image's device" % cap)
+        nws = int(L.pysp_jpeg_rgb_workspace_bytes(H, W, s))
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        n = torch.empty((), dtype=torch.int64, device=dev)
+        _capi.check(L.pysp_jpeg_encode_rgb(rgb.data_ptr(), rgb.stride(0), H, W, int(quality), s, out_tensor.data_ptr(),
+                                           out_tensor.numel(), n.data_ptr(), ws.data_ptr(), nws, _stream_ptr(stream)))
+    return out_tensor, n
+
+
 def normalize(raw, black, white, stream=None):
     """bayer_normalize on the device: uint16 [H,W] -> float32 [H,W]."""
     require_cuda()

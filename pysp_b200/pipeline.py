@@ -12,7 +12,9 @@ three planes of it), so one copy moves a frame.
 With out="jpeg" each frame is developed into device ycc420 planes and encoded on the device (engine.encode_jpeg, quality
 `jpeg_quality`); its length goes to pinned host memory, and once that has landed exactly that many bytes are copied into the
 frame's output.  The host waits for frame i's length only after frame i + depth - 1 has been queued, so the later frames' work
-keeps the GPU busy while it waits.  `run` returns the lengths.
+keeps the GPU busy while it waits.  `run` returns the lengths.  `jpeg_subsampling` "4:4:4" or "4:2:2" (or Pillow's 0 / 1)
+develops srgb_u8 into the slot's device buffer instead and encodes that with engine.encode_jpeg_rgb; the default "4:2:0"
+keeps the ycc420 planes route.
 """
 import torch
 
@@ -21,15 +23,17 @@ from . import engine
 
 class FramePipeline:
     def __init__(self, height, width, wb, cam_to_srgb, stages=1, pattern="RGGB", black=None, white=None,
-                 hdr=False, gamma=False, out="lin", device=None, depth=3, jpeg_quality=75):
+                 hdr=False, gamma=False, out="lin", device=None, depth=3, jpeg_quality=75, jpeg_subsampling="4:2:0"):
         engine.require_cuda()
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         self.h, self.w = int(height), int(width)
         self.jpeg = out == "jpeg"
         self.jpeg_quality = int(jpeg_quality)
-        planes = out in ("ycc420", "jpeg")
+        self.jpeg_subsampling = engine.jpeg_subsampling(jpeg_subsampling)
+        self.jpeg_rgb = self.jpeg and self.jpeg_subsampling != engine._capi.JPEG_420     # 4:4:4 / 4:2:2 from srgb_u8
+        planes = out == "ycc420" or (self.jpeg and not self.jpeg_rgb)
         self.kw = dict(wb=wb, cam_to_srgb=cam_to_srgb, stages=stages, pattern=pattern, black=black, white=white,
-                       hdr=hdr, gamma=gamma, out="ycc420" if self.jpeg else out)
+                       hdr=hdr, gamma=gamma, out=("srgb_u8" if self.jpeg_rgb else "ycc420") if self.jpeg else out)
         self.out_dtype = engine._OUT_DTYPES[engine._OUT_KINDS[self.kw["out"]]]
         self.out_shape = (engine.i420_bytes(self.h, self.w),) if planes else (self.h, self.w, 3)
         self.depth = depth
@@ -40,7 +44,8 @@ class FramePipeline:
         # what develop writes into: the output tensor itself, or the three planes over the flat I420 buffer
         self.d_dst = [engine.i420_planes(d, self.h, self.w) if planes else d for d in self.d_out]
         if self.jpeg:
-            self.jpeg_bytes = engine.jpeg_max_bytes(self.h, self.w)
+            self.jpeg_bytes = (engine.jpeg_rgb_max_bytes(self.h, self.w, self.jpeg_subsampling) if self.jpeg_rgb
+                               else engine.jpeg_max_bytes(self.h, self.w))
             with torch.cuda.device(self.device):
                 self.d_jpeg = [torch.empty(self.jpeg_bytes, dtype=torch.uint8, device=self.device) for _ in range(depth)]
 
@@ -48,7 +53,8 @@ class FramePipeline:
         return torch.empty((self.h, self.w), dtype=torch.int16).pin_memory()
 
     def pinned_output(self):
-        """a host buffer for one output; for out="jpeg" sized to the largest file (engine.jpeg_max_bytes)"""
+        """a host buffer for one output; for out="jpeg" sized to the largest file (engine.jpeg_max_bytes, or
+        engine.jpeg_rgb_max_bytes for 4:4:4 / 4:2:2)"""
         if self.jpeg:
             return torch.empty(self.jpeg_bytes, dtype=torch.uint8).pin_memory()
         return torch.empty(self.out_shape, dtype=self.out_dtype).pin_memory()
@@ -95,7 +101,11 @@ class FramePipeline:
                 with torch.cuda.stream(s):
                     self.d_in[k].copy_(src, non_blocking=True)
                     engine.develop(self.d_in[k], out_tensor=self.d_dst[k], stream=s, **self.kw)
-                    _, n = engine.encode_jpeg(self.d_dst[k], self.jpeg_quality, out_tensor=self.d_jpeg[k], stream=s)
+                    if self.jpeg_rgb:
+                        _, n = engine.encode_jpeg_rgb(self.d_dst[k], self.jpeg_quality, self.jpeg_subsampling,
+                                                      out_tensor=self.d_jpeg[k], stream=s)
+                    else:
+                        _, n = engine.encode_jpeg(self.d_dst[k], self.jpeg_quality, out_tensor=self.d_jpeg[k], stream=s)
                     lens[i].copy_(n, non_blocking=True)
                     landed[i] = torch.cuda.Event()
                     landed[i].record(s)
